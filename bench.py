@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # reference CPU path (restated)
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's results to DIR/*.npy
 
 Workload at N=1 = BASELINE.json configs[1]: 1,024 independent horizon-24
 lower-level MPC QPs (512 small-EV + 512 large-EV), inputs drawn as the
@@ -43,6 +44,7 @@ PKG = os.path.join(ROOT, "incentive-design-mpc_b200")
 for p in (ROOT, PKG):
     if p not in sys.path:
         sys.path.insert(0, p)
+sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 N_HORIZON = 24
 METRIC = "lompc_qp_solves_per_sec"
@@ -149,11 +151,7 @@ def run_reference(args, rank: int, world: int) -> None:
     work = draw_workload(args.batch, N_HORIZON, 2)
     for _ in range(max(args.warmup, 1)):
         used = cpu_pass(work, N_HORIZON)
-    # bound the whole run to a few minutes
-    t0 = time.perf_counter()
-    cpu_pass(work, N_HORIZON)
-    one = time.perf_counter() - t0
-    steps = max(1, min(args.steps, int(120.0 / max(one, 1e-9))))
+    steps = args.steps
     t0 = time.perf_counter()
     for _ in range(steps):
         cpu_pass(work, N_HORIZON)
@@ -307,6 +305,7 @@ def run_ours(args, rank: int, local_rank: int, world: int) -> None:
     launches = per_replay
     dev_ms = e_start.elapsed_time(e_stop)
     assert int(out_blocks[:K].view(torch.int64)[:, 0].remainder(4).max()) == 0, "a QP inside the timed region failed"
+    last_block = out_blocks[K - 1].cpu().numpy() if args.dump_outputs else None  # the last timed step's out block
 
     # ---- the same K steps with independent steps allowed to OVERLAP: the batches of different steps have nothing to
     # do with each other, and one 1,024-QP launch (256 single-warp CTAs) leaves most of the GPU idle, so a caller with
@@ -376,6 +375,7 @@ def run_ours(args, rank: int, local_rank: int, world: int) -> None:
     torch.cuda.synchronize()
     e2e_s = time.perf_counter() - t0
     barrier()
+    e2e_last = [(w.copy(), c.copy()) for w, c in zip(sset.w, sset.cost)] if args.dump_outputs else None
 
     # saturating batch (explains `value`: 1,024 QPs cannot fill 148 SMs)
     sat = None
@@ -476,9 +476,29 @@ def run_ours(args, rank: int, local_rank: int, world: int) -> None:
         }
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline_leg(args)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, sset, evs_order, last_block, e2e_last)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(path, sset, evs_order, last_block, e2e_last):
+    """Writes what the timed steps returned in their last step as float64 DIR/<name>.npy, so that two builds can be
+    compared output for output (the inputs are seeded): `step_*` is the out block of the device-timed leg's last
+    step (w [B, N] and cost [B] of every EV type, and the worst QP status of the launch), `e2e_*` the w / cost views
+    of the set after the last end-to-end step (the seeded workload)."""
+    os.makedirs(path, exist_ok=True)
+    out = {"step_worst_status": np.array([last_block[:8].view(np.int64)[0] % 4])}
+    f64 = last_block.view(np.float64)
+    for i, ev in enumerate(evs_order):
+        B, N = sset.batch_sizes[i], sset.N
+        o_w, o_cost = sset.offsets(i)[3:]
+        out[f"step_w_{ev}"] = f64[o_w // 8: o_w // 8 + B * N].reshape(B, N)
+        out[f"step_cost_{ev}"] = f64[o_cost // 8: o_cost // 8 + B]
+        out[f"e2e_w_{ev}"], out[f"e2e_cost_{ev}"] = e2e_last[i]
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def saturated_run(solvers, dev, rank, fp64_peak):
@@ -708,7 +728,7 @@ def cpu_baseline_leg(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="timed steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=1024, help="QPs per GPU per step (configs[1]: 1024)")
@@ -720,7 +740,13 @@ def main():
     ap.add_argument("--closed-loop-chain", default="reference", choices=["reference", "partition"])
     ap.add_argument("--sharded-iters", type=int, default=200,
                     help="price iterations of the configs[2] leg (65,536 EVs sharded over the ranks; 0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the CUDA path (--impl ours)")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
