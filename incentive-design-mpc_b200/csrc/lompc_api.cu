@@ -245,8 +245,6 @@ int launch_solve(const lompc_handle* h, const lompc::SolveArgs& a, cudaStream_t 
     if (N == 24) return launch_solve_reg_variant<24, NSEG>(h, a, stream);
     if (N == 12) return launch_solve_reg_variant<12, NSEG>(h, a, stream);
   }
-  // Threads per block: as many as fit the 227 KB of shared memory, capped at 128;
-  // small batches use small blocks so that more SMs take part.
   // Threads per block: the size that keeps most warps resident per SM (shared memory is the limit: 6-7 vectors of
   // N doubles per QP), capped at 128; small batches use small blocks so that more SMs take part.
   int T = 32;
@@ -262,6 +260,10 @@ int launch_solve(const lompc_handle* h, const lompc::SolveArgs& a, cudaStream_t 
     }
   }
   while (T > 32 && (a.B + T - 1) / T < 148) T >>= 1;
+  // Horizons whose columns do not fit 32 threads (N > 129 large EV, N > 151 small EV): the largest power of two that
+  // fits.  The kernel has no barrier and its layout is [k*T + t], so any T works; at T = 1 every N <= 4096 fits.
+  // (The throughput of these partial-warp CTAs has not been measured.)
+  while (T > 1 && lompc::SmemLayout<NSEG>::bytes(N, T) > 227 * 1024) T >>= 1;
   const size_t smem = lompc::SmemLayout<NSEG>::bytes(N, T);
   if (smem > 227 * 1024) return LOMPC_ERR_ARG;
   static std::atomic<uint64_t> configured{0};  // per device ordinal (the attribute is per context)
@@ -647,6 +649,8 @@ inline unsigned nblk(int64_t n, int t) { return (unsigned)((n + t - 1) / t); }
 int launch_group_step(const lompc_handle* h, const lompc::PriceArgs& p, int it, cudaStream_t s) {
   const int N = h->cs.N, wpc = 2;
   const size_t smem = (size_t)wpc * (lompc::price_step_scratch_doubles(N, p.r) + (p.r + 7) / 8) * sizeof(double);
+  // the scratch of two warps grows with N: above N ~ 750 it exceeds the shared-memory opt-in (not a CUDA failure)
+  if (smem > 227 * 1024) return LOMPC_ERR_ARG;
   // (the horizons of the closed loop and of BASELINE configs[2] get the unrolled recursions of the price step)
   if (N == 24) {
     lompc::group_step_kernel<24><<<nblk(p.G, wpc), 32 * wpc, smem, s>>>(h->cs, p, it);

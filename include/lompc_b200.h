@@ -67,7 +67,8 @@ int lompc_set_options(lompc_t* h, int max_iter, double tol);
 /* Kernel choice: 0 = automatic (register-resident kernel for N = 12, 24 - 64 threads x 4 CTAs per SM; large EV
  * on grids that fill the GPU: one 256-thread CTA per SM; plain batches of >= 65,536 QPs at N = 24: the same
  * kernel with bulk-copied rows, see 9 - and the any-N shared-memory kernel otherwise),
- * 1 = always the any-N kernel, 4 / 7 = one register-kernel shape regardless of the batch size (4 = 64 threads x
+ * 1 = always the any-N kernel (every N that lompc_create accepts, 1..4096: up to 128 threads per CTA, fewer where
+ * N's columns do not fit - below 32 threads above N = 129 large EV / 151 small EV, down to one thread at N = 4096), 4 / 7 = one register-kernel shape regardless of the batch size (4 = 64 threads x
  * 4 CTAs per SM, 7 = 256 x 1; the other shapes of round 1's sweep are no longer compiled: LOMPC_ERR_ARG);
  * 8 = the warp-cooperative latency kernel (one QP per group of N/3 lanes, time-parallel sweeps; N = 12, 24,
  * 48, 96), which automatic mode picks for batches too small to fill the GPU with one QP per thread;
