@@ -74,6 +74,7 @@ SIGNATURES = {
     "price_last_cycles": (C.c_int64, [C.c_void_p, C.c_int]),
     "price_debug_force_nnqp_fallback": (C.c_int, [C.c_int]),
     "price_debug_pivot_pool": (C.c_int, [C.c_int]),
+    "price_debug_record_errors": (C.c_int, [C.c_void_p, C.c_void_p]),
     "price_debug_force_compact_step": (C.c_int, [C.c_int]),
     "price_shard_begin": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                     C.c_int, C.c_int, C.c_int, C.c_double, C.c_double] + [C.c_void_p] * 10 +

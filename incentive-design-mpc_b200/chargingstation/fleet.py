@@ -34,7 +34,7 @@ import numpy as np
 from chargingstation import _native
 from chargingstation.bimpc import BiMPC
 from chargingstation.charging_station import ChargingStationConstants, partition_edges
-from chargingstation.price_solver import PriceSolver
+from chargingstation.price_solver import PriceSolver, tol_type_max
 from chargingstation.settings import (MAX_INITIAL_SOC, MAX_PRICE_SOLVER_ITERATIONS, MIN_FULL_CHARGE_FRACTION,
                                       MIN_INITIAL_SOC, PRICE_SOLVER_TOL_TYPE)
 
@@ -42,10 +42,12 @@ from chargingstation.settings import (MAX_INITIAL_SOC, MAX_PRICE_SOLVER_ITERATIO
 class ChargingStationFleet:
     def __init__(self, consts: ChargingStationConstants, nstations: int, demand: np.ndarray | None = None,
                  seed: int = 0, rng: str = "device", chain: str = "reference", device: int = 0,
-                 max_price_iter: int = MAX_PRICE_SOLVER_ITERATIONS) -> None:
+                 max_price_iter: int = MAX_PRICE_SOLVER_ITERATIONS, tol_type: str | None = None) -> None:
         """
         consts:     the station's constants (every station shares them); ``consts.demand`` is
                     used for all stations unless ``demand`` [S, >= Tf + N_bi + 1] is given.
+        tol_type:   convergence test of the price loops, "avg" or "max" (price_solver.py:121-128);
+                    None = PRICE_SOLVER_TOL_TYPE.
         """
         import torch
         assert rng in ("device", "numpy") and chain in ("reference", "partition")
@@ -61,6 +63,8 @@ class ChargingStationFleet:
         self.r = 2 * self.N_lo if consts.price_type == "linear" else 3 * self.N_lo
         self.rng_mode, self.chain, self.seed = rng, chain, int(seed)
         self.max_price_iter = int(max_price_iter)
+        self.tol_type = tol_type
+        tol_type_max(tol_type, PRICE_SOLVER_TOL_TYPE)  # rejects anything but "avg", "max" and None here
         S, M, P, N_lo, N_bi = self.S, self.M, self.P, self.N_lo, self.N_bi
         if demand is None:
             demand = np.broadcast_to(consts.demand, (S, consts.demand.shape[0]))
@@ -150,7 +154,7 @@ class ChargingStationFleet:
         S, M, P, N_lo, N_bi, t = self.S, self.M, self.P, self.N_lo, self.N_bi, self.t
         G, B = P * S, S * M
         lmbd_r = 0.0  # charging_station.py:162
-        tol_max = 1 if PRICE_SOLVER_TOL_TYPE == "max" else 0
+        tol_max = tol_type_max(self.tol_type, PRICE_SOLVER_TOL_TYPE)
         marks = []
 
         def mark(name):

@@ -23,6 +23,17 @@ from chargingstation.settings import (MAX_PRICE_SOLVER_ITERATIONS,
 from chargingstation import settings
 
 
+def tol_type_max(tol_type: str | None, default: str) -> int:
+    """The C ABI's tol_type_max flag for a tolerance type of the price loop's convergence test
+    (settings.PRICE_SOLVER_TOL_TYPE, price_solver.py:121-128): "avg" (error of the mean response) or "max" (largest
+    error of a single EV).  None takes ``default``, the module constant, as the reference does."""
+    if tol_type is None:
+        return 1 if default == "max" else 0
+    if tol_type not in ("avg", "max"):
+        raise ValueError(f'tol_type must be "avg" or "max", not {tol_type!r}')
+    return 1 if tol_type == "max" else 0
+
+
 class PriceSolver:
     def __init__(self, N: int, consts: LoMPCConstants, price_type: str, device: int = 0) -> None:
         """
@@ -249,14 +260,16 @@ class PriceSolver:
 
     # ------------------------------------------------------- batched extension
     def compute_optimal_prices_batch(self, group_off, y0, w_ref, lmbd_r, prev_prices, history: bool = False,
-                                     max_iter: int = MAX_PRICE_SOLVER_ITERATIONS):
+                                     max_iter: int = MAX_PRICE_SOLVER_ITERATIONS, tol_type: str | None = None):
         """``compute_optimal_prices`` for G groups at once.
 
         group_off: int32 [G+1], EVs sorted by group.  y0: [B] SoCs.  w_ref: [G, N].
         lmbd_r: [G].  prev_prices: [G, 3N] warm start (zero padded for "linear").
+        tol_type: "avg" or "max" (the convergence test, price_solver.py:121-128); None = PRICE_SOLVER_TOL_TYPE.
         Returns (prices [G, 3N] numpy, stats dict of arrays: iter, price_before_reg,
         price_after_reg, w_k [G, N], total_iters; with ``history`` also hist_ac /
         hist_pred [G, cap])."""
+        tol_max = tol_type_max(tol_type, PRICE_SOLVER_TOL_TYPE)
         torch, dev = self._torch()
         N = self.N
         group_off = np.ascontiguousarray(group_off, dtype=np.int32)
@@ -280,7 +293,7 @@ class PriceSolver:
         total = C.c_int32(0)
         rc = self._lib.price_solve_dev(
             self._h, G, B, off_d.data_ptr(), y0_d.data_ptr(), w_ref_d.data_ptr(), lr_d.data_ptr(), self.r,
-            int(max_iter), 1 if PRICE_SOLVER_TOL_TYPE == "max" else 0, float(self.eps_reg), float(self.eps_tol),
+            int(max_iter), tol_max, float(self.eps_reg), float(self.eps_tol),
             prices.data_ptr(), iters.data_ptr(), pre.data_ptr(), post.data_ptr(), w_k.data_ptr(),
             hist_ac.data_ptr() if history else None, hist_pred.data_ptr() if history else None, cap,
             C.byref(total), self._stream())

@@ -454,6 +454,13 @@ int price_debug_pivot_pool(int slots) {
   return LOMPC_OK;
 }
 
+int price_debug_record_errors(double* w_err_max, double* w_avg_err) {
+  if (!w_err_max != !w_avg_err) return LOMPC_ERR_ARG;
+  CK(cudaMemcpyToSymbol(lompc::g_record_err_max, &w_err_max, sizeof(double*)));
+  CK(cudaMemcpyToSymbol(lompc::g_record_err_avg, &w_avg_err, sizeof(double*)));
+  return LOMPC_OK;
+}
+
 int64_t price_last_cycles(const lompc_t* h, int which) {
   if (h && which == 5) return h->last_pivot_overflows;
   if (h && which == 6) return h->last_nnqp_cap_hits;
@@ -1215,35 +1222,41 @@ int launch_fused(lompc_handle* h, const lompc::FusedArgs& a, cudaStream_t s) {
   return LOMPC_OK;
 }
 
-// The parametric loop (lompc_price_warp.cuh): one warp per group / per station.
+// The parametric loop (lompc_price_warp.cuh): one warp per group / per station; the "max" tolerance type has its own
+// instantiation.
 template <int N>
 int launch_fused_warp(lompc_handle* h, const lompc::FusedArgs& a, cudaStream_t s) {
   constexpr size_t smem = lompc::WarpLoopSmem<N>::bytes;
   static_assert(smem <= 48 * 1024, "no shared-memory opt-in needed");
-  if (a.chain_P > 0)
-    lompc::price_station_chain_warp_kernel<N><<<(unsigned)a.chain_S, 32, smem, s>>>(h->cs, a);
-  else
-    lompc::price_group_warp_kernel<N><<<(unsigned)a.G, 32, smem, s>>>(h->cs, a);
+  if (a.tol_type_max) {
+    if (a.chain_P > 0)
+      lompc::price_station_chain_warp_kernel<N, true><<<(unsigned)a.chain_S, 32, smem, s>>>(h->cs, a);
+    else
+      lompc::price_group_warp_kernel<N, true><<<(unsigned)a.G, 32, smem, s>>>(h->cs, a);
+  } else if (a.chain_P > 0) {
+    lompc::price_station_chain_warp_kernel<N, false><<<(unsigned)a.chain_S, 32, smem, s>>>(h->cs, a);
+  } else {
+    lompc::price_group_warp_kernel<N, false><<<(unsigned)a.G, 32, smem, s>>>(h->cs, a);
+  }
   COUNT_LAUNCH();
   CK(cudaGetLastError());
   return LOMPC_OK;
 }
 
 // Is there a device-resident loop for this handle?  N = 12, 24: the parametric and the thread-per-EV kernels; N = 48,
-// 96: the parametric kernel only ("avg" tolerance type, loop mode 0 or 2).  Otherwise: the phase-split loop.
-inline bool has_fused_loop(const lompc_handle* h, int tol_type_max) {
+// 96: the parametric kernel only (loop mode 0 or 2).  Otherwise: the phase-split loop.  Both tolerance types alike.
+inline bool has_fused_loop(const lompc_handle* h) {
   if (h->variant == 1 || h->loop_mode == 1) return false;
   const int N = h->cs.N;
   if (N == 12 || N == 24) return true;
-  return (N == 48 || N == 96) && !tol_type_max && (h->loop_mode == 2 || (h->loop_mode == 0 && kParametricLoopByDefault));
+  return (N == 48 || N == 96) && (h->loop_mode == 2 || (h->loop_mode == 0 && kParametricLoopByDefault));
 }
 
 // compute_optimal_prices for whole groups resident on this GPU: one CTA per group, no host loop.
 int price_solve_fused(lompc_handle* h, const lompc::FusedArgs& a, cudaStream_t s) {
   const int N = h->cs.N;
-  // loop mode 2 = the parametric one-warp-per-group loop ("avg" tolerance type), 3 = the thread-per-EV loop;
-  // 0 = automatic
-  const bool parametric = !a.tol_type_max && (h->loop_mode == 2 || (h->loop_mode == 0 && kParametricLoopByDefault));
+  // loop mode 2 = the parametric one-warp-per-group loop, 3 = the thread-per-EV loop; 0 = automatic
+  const bool parametric = h->loop_mode == 2 || (h->loop_mode == 0 && kParametricLoopByDefault);
   if (parametric) {
     if (N == 24) return launch_fused_warp<24>(h, a, s);
     if (N == 12) return launch_fused_warp<12>(h, a, s);
@@ -1327,7 +1340,7 @@ int price_solve_dev(lompc_t* h, int32_t G, int64_t B, const int32_t* group_off, 
   if (total_iters) *total_iters = 0;
   if (G == 0) return LOMPC_OK;
   CK(cudaSetDevice(h->device));
-  if (has_fused_loop(h, tol_type_max))
+  if (has_fused_loop(h))
     return price_solve_fused_entry(h, G, B, group_off, y0, w_ref, lmbd_r, r, max_iter, tol_type_max, eps_reg, eps_tol,
                                    prices, iters, price_pre, price_post, w_k_out, hist_ac, hist_pred, hist_cap,
                                    total_iters, 0, 0, nullptr, nullptr, stream);
@@ -1390,7 +1403,7 @@ int price_solve_chain_dev(lompc_t* h, int32_t S, int32_t P, int64_t B, const int
     return LOMPC_ERR_ARG;
   if (max_group_iters) *max_group_iters = 0;
   CK(cudaSetDevice(h->device));
-  if (!has_fused_loop(h, tol_type_max)) {
+  if (!has_fused_loop(h)) {
     // no fused kernel for this horizon: the same chain as P phase-split loops, one per partition slice
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const int N = h->cs.N;

@@ -37,8 +37,26 @@ namespace lompc {
 // Test hook: pivot slots the parametric loop may use (price_debug_pivot_pool(); 32 = all).  A small pool makes the
 // direct jobs of group_loop_warp, which a full pool needs about once in 10^4 groups, the common case.
 __device__ int g_pivot_pool = 32;
+// Test hook: [G] device arrays (price_debug_record_errors()) that receive, per group, w_err_max and w_avg_err of the
+// last convergence test of a parametric "max" loop; NULL = off.
+__device__ double* g_record_err_max = nullptr;
+__device__ double* g_record_err_avg = nullptr;
 constexpr int kMaxPivots = 32;  // solved EVs kept at a time (3 permanent: lowest gamma, virtual, highest gamma)
 constexpr int kQueueCap = 64;   // intervals between neighbouring pivots waiting for their verdict
+
+// A-bar-norm of w - w_ref (price_solver.py:207), w = wa + t (wb - wa): the formula and summation order of the
+// thread-per-EV loop (lompc_price_fused.cuh), so that a solved EV (t = 0) gives the same error there and here.
+template <int N>
+__device__ __forceinline__ double ev_err_warp(const double* wa, const double* wb, const double t, const double* wref,
+                                              const double kappa) {
+  double cum = 0.0, e2 = 0.0;
+  for (int k = 0; k < N; ++k) {
+    const double v = wa[k] + t * (wb[k] - wa[k]) - wref[k];
+    cum += v;
+    e2 += cum * cum + kappa * v * v;
+  }
+  return sqrt(e2);
+}
 
 template <int N>
 struct WarpLoopSmem {
@@ -60,7 +78,12 @@ struct WarpLoopSmem {
 // loop's horizons) and 48, 96 (configs[4]'s: 16 / 32 lanes per QP, 2 / 1 QPs per warp pass).
 // Scratch in global memory (a.w_scratch rows b0 .., N doubles per EV): the sorted gammas and their
 // prefix sums (2n + 1 doubles; the launcher sizes the rows so that this fits for every n >= 1).
-template <int N, int NSEG>
+// MAXTOL: the "max" tolerance type (price_solver.py:121-128), the largest error of a single EV.  Within a critical
+// region w is affine in gamma, so the error is convex in gamma on every interpolated interval and its largest value
+// over the interval's EVs is at the first or the last of them: the maximum over the group is the maximum over the real
+// EVs solved (pivots, direct jobs) and those two EVs of every interpolated interval.  The virtual EV is not an EV of
+// the group and never enters it.  A separate instantiation, so that the "avg" kernels carry none of this code.
+template <int N, int NSEG, bool MAXTOL>
 __device__ __forceinline__ bool group_loop_warp(const Consts& cs, const FusedArgs& a, const int g, double* smem,
                                                 const double* p_in, double* p_out, double* p_out2) {
   constexpr int SPL = 3, LPQ = N / SPL, QPW = 32 / LPQ;
@@ -182,6 +205,7 @@ __device__ __forceinline__ bool group_loop_warp(const Consts& cs, const FusedArg
     double wsum[NW];  // lane l, slot u: sum over the group's EVs of w_i[l + 32 u]
 #pragma unroll
     for (int u = 0; u < NW; ++u) wsum[u] = 0.0;
+    [[maybe_unused]] double emax = 0.0;  // MAXTOL: largest EV error this lane has evaluated in this pass
     // direct job: EVs [dj_first, dj_first + dj_cnt) of an interval (dj_sa, dj_sb) that found no free pivot slots are
     // solved one by one into the (idle) price-step scratch - exact, just without the saving
     int dj_first = 0, dj_cnt = 0, dj_sa = 0, dj_sb = 0;
@@ -238,6 +262,20 @@ __device__ __forceinline__ bool group_loop_warp(const Consts& cs, const FusedArg
           if (lane == 0) atomicAdd(a.flags + 3, 1);
         }
         __syncwarp();
+        if constexpr (MAXTOL) {  // one solved EV per lane: the direct job's rows, or the real EVs of the batch
+          int sv = -1;
+          if (direct) {
+            if (lane < q) sv = lane;
+          } else {
+            int t = 0;
+            for (unsigned m = batch & ~2u; m; m &= m - 1, ++t)
+              if (t == lane) sv = __ffs(m) - 1;
+          }
+          if (sv >= 0) {
+            const double* w = direct ? WS + sv * N : PW + sv * N;
+            emax = fmax(emax, ev_err_warp<N>(w, w, 0.0, WREF, kappa));
+          }
+        }
         if (direct) {
           for (int t = 0; t < q; ++t)
 #pragma unroll
@@ -291,6 +329,13 @@ __device__ __forceinline__ bool group_loop_warp(const Consts& cs, const FusedArg
                 const double wa = PW[sa * N + lane + 32 * u], wb = PW[sb * N + lane + 32 * u];
                 wsum[u] += cnt * wa + coef * (wb - wa);
               }
+            if constexpr (MAXTOL) {  // the interval's first (lane 0) and last (lane 1) EV, on the interpolant
+              if (lane < 2) {
+                const double gi = GS[lane == 0 ? fa : lb];
+                emax = fmax(emax, ev_err_warp<N>(PW + sa * N, PW + sb * N, gb > ga ? (gi - ga) / (gb - ga) : 0.0,
+                                                 WREF, kappa));
+              }
+            }
           }
           release(sa);
           release(sb);
@@ -363,6 +408,10 @@ __device__ __forceinline__ bool group_loop_warp(const Consts& cs, const FusedArg
     flag = 0;
     const long long t_b = clock64();
     cyc_qp += t_b - t_a;
+    if constexpr (MAXTOL) {
+#pragma unroll
+      for (int d = 16; d >= 1; d >>= 1) emax = fmax(emax, __shfl_xor_sync(full, emax, d));
+    }
     if (lane == 0) {
       const double cost_sc = SC[0];
       if (it > 0 && a.hist_ac && it - 1 < a.hist_cap) {  // price_solver.py:135-139
@@ -375,8 +424,15 @@ __device__ __forceinline__ bool group_loop_warp(const Consts& cs, const FusedArg
       } else {
         double w_avg_err, w0_err;
         price_errors(N, kappa, WSUM, (double)n, WREF, w_avg_err, w0_err);
-        if (w_avg_err <= tolg) flag = 1;  // price_solver.py:125 ("avg" tolerance type)
-
+        if constexpr (MAXTOL) {
+          if (emax <= tolg) flag = 1;  // price_solver.py:125 ("max" tolerance type)
+          if (g_record_err_max) {
+            g_record_err_max[g] = emax;
+            g_record_err_avg[g] = w_avg_err;
+          }
+        } else {
+          if (w_avg_err <= tolg) flag = 1;  // price_solver.py:125 ("avg" tolerance type)
+        }
       }
     }
     flag = __shfl_sync(full, flag, 0);
@@ -428,22 +484,22 @@ __device__ __forceinline__ bool group_loop_warp(const Consts& cs, const FusedArg
   return true;
 }
 
-// Grid = the groups: one warp (= one CTA) per group.
-template <int N>
+// Grid = the groups: one warp (= one CTA) per group.  MAXTOL = "max" tolerance type (a.tol_type_max).
+template <int N, bool MAXTOL>
 __global__ void __launch_bounds__(32, LOMPC_CHAIN_MINB) price_group_warp_kernel(const __grid_constant__ Consts cs,
                                                                  const __grid_constant__ FusedArgs a) {
   extern __shared__ double smem[];
   const int g = blockIdx.x;
   double* row = a.prices + (size_t)g * 3 * N;
   if (cs.large)
-    group_loop_warp<N, 4>(cs, a, g, smem, row, row, nullptr);
+    group_loop_warp<N, 4, MAXTOL>(cs, a, g, smem, row, row, nullptr);
   else
-    group_loop_warp<N, 1>(cs, a, g, smem, row, row, nullptr);
+    group_loop_warp<N, 1, MAXTOL>(cs, a, g, smem, row, row, nullptr);
 }
 
 // Grid = the stations: one warp per station walks its P partitions in the reference's warm-start order
 // (see price_station_chain_kernel in lompc_price_fused.cuh).
-template <int N>
+template <int N, bool MAXTOL>
 __global__ void __launch_bounds__(32, LOMPC_CHAIN_MINB) price_station_chain_warp_kernel(const __grid_constant__ Consts cs,
                                                                          const __grid_constant__ FusedArgs a) {
   extern __shared__ double smem[];
@@ -452,8 +508,8 @@ __global__ void __launch_bounds__(32, LOMPC_CHAIN_MINB) price_station_chain_warp
   for (int p = 0; p < a.chain_P; ++p) {
     const int g = p * S + s;
     double* row = a.prices + (size_t)g * 3 * N;
-    const bool solved = cs.large ? group_loop_warp<N, 4>(cs, a, g, smem, prev, prev, row)
-                                 : group_loop_warp<N, 1>(cs, a, g, smem, prev, prev, row);
+    const bool solved = cs.large ? group_loop_warp<N, 4, MAXTOL>(cs, a, g, smem, prev, prev, row)
+                                 : group_loop_warp<N, 1, MAXTOL>(cs, a, g, smem, prev, prev, row);
     if (!solved)
       for (int k = threadIdx.x; k < 3 * N; k += 32) row[k] = 0.0;
     __syncwarp();

@@ -231,8 +231,8 @@ int price_solve_dev(lompc_t* h, int32_t G, int64_t B, const int32_t* group_off, 
  * warm start (in: PriceSolver.prev_prices of every station, out: the same after the step);
  * prices[P*S,3N] receives every group's regularised prices (zeros for an empty group,
  * charging_station.py:270; its iters = -1).  One CTA per station runs its P loops back to back, so
- * stations do not wait for each other (N = 12, 24; other horizons run the same chain as P phase-split
- * loops, one per partition slice).  station_order[S] (may be NULL) = a permutation of the stations:
+ * stations do not wait for each other (N = 12, 24; N = 48, 96 with the parametric loop; otherwise the same
+ * chain runs as P phase-split loops, one per partition slice).  station_order[S] (may be NULL) = a permutation of the stations:
  * the order in which CTAs pick them up (longest expected chains first shortens the tail).
  * Synchronises; max_group_iters = length of the longest loop.                                       */
 int price_solve_chain_dev(lompc_t* h, int32_t S, int32_t P, int64_t B, const int32_t* group_off, const double* y0,
@@ -242,12 +242,14 @@ int price_solve_chain_dev(lompc_t* h, int32_t S, int32_t P, int64_t B, const int
                           int32_t* max_group_iters, void* stream);
 
 /* price_solve_dev / price_solve_chain_dev run, for the compiled horizons (N = 12, 24; N = 48, 96 with the parametric
- * loop and the "avg" tolerance type), ONE kernel that iterates every group to convergence on the device.  Loop modes: 0 = automatic; 1 = the phase-split loop below (any N; the
- * path a multi-GPU caller drives); 2 = the PARAMETRIC loop, one warp per group: the EVs of a group differ only in
- * gamma and the QP's solution is piecewise affine in it, so only the extreme EVs, the virtual EV (gamma_sc) and the
- * EVs that bracket a change of active set are solved and the rest is interpolated (SURVEY.md 8 row f3; "avg"
- * tolerance type, price_solver.py:196-214); 3 = the thread-per-EV loop, one CTA per group.  All give the same
- * iteration counts and prices up to rounding.  price_last_qp_solves = LoMPC QPs solved by the last fused call;
+ * loop), ONE kernel that iterates every group to convergence on the device, for either tolerance type.  Loop modes:
+ * 0 = automatic (the parametric loop); 1 = the phase-split loop below (any N; the path a multi-GPU caller drives);
+ * 2 = the PARAMETRIC loop, one warp per group: the EVs of a group differ only in gamma and the QP's solution is
+ * piecewise affine in it, so only the extreme EVs, the virtual EV (gamma_sc) and the EVs that bracket a change of
+ * active set are solved and the rest is interpolated (SURVEY.md 8 row f3; price_solver.py:196-214 - for "max" the
+ * error of an interpolated stretch of EVs is convex in gamma, so its largest value is at the stretch's first or last
+ * EV); 3 = the thread-per-EV loop, one CTA per group (N = 12, 24; the phase-split loop at other horizons).  All give
+ * the same iteration counts and prices up to rounding.  price_last_qp_solves = LoMPC QPs solved by the last fused call;
  * price_last_cycles(h, 5) = groups of the last parametric call whose pool of 32 pivot slots ran out (about one group in
  * 10^4 on a fleet's first step; the EVs of the stuck intervals are then solved one by one: exact, informational),
  * price_last_cycles(h, 6) = groups of the last device-resident call whose price step (price_solver.py:216-246) ended
@@ -257,13 +259,17 @@ int price_solve_chain_dev(lompc_t* h, int32_t S, int32_t P, int64_t B, const int
  * price_last_cycles(h, 8) = groups that took the fallback (informational).
  * price_debug_force_nnqp_fallback: test hook - non-zero sends EVERY price step of the current device through the
  * fallback (the parity tests of the price loop are run both ways); price_debug_pivot_pool: test hook - the pivot
- * slots the parametric loop may use (4..32, default 32), so that a test can make slot shortage the common case. */
+ * slots the parametric loop may use (4..32, default 32), so that a test can make slot shortage the common case;
+ * price_debug_record_errors: test hook - while set (both non-NULL: device arrays [G] of the current device; both NULL:
+ * off), every group of a parametric "max" loop writes the w_err_max and w_avg_err of its last convergence test
+ * (price_solver.py:196-214).  With max_iter = 1 these are the errors at the warm-start prices. */
 int price_set_loop_mode(lompc_t* h, int mode);
 int64_t price_last_qp_solves(const lompc_t* h);
 /* SM cycles of the last fused call summed over groups: which = 0 LoMPC passes, 1 price steps. */
 int64_t price_last_cycles(const lompc_t* h, int which);
 int price_debug_force_nnqp_fallback(int on);
 int price_debug_pivot_pool(int slots);
+int price_debug_record_errors(double* w_err_max, double* w_avg_err);
 /* Test hook: non-zero makes every device-resident loop take the code path of fleet-scale launches (the compact price
  * step: recursions unrolled 4 stages per trip; automatic from 1,184 groups / stations per launch). */
 int price_debug_force_compact_step(int on);
