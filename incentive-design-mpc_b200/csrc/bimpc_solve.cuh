@@ -328,8 +328,13 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
   // decoupled from the rest of the program and its optimum is w_q = 0: it is left out of the
   // Newton system (the block size 2P+1 shrinks to active+1; early in a simulation only a third
   // of the partitions is populated).  Thread 0 builds the compact list.
+  // It also checks that every input is finite: a NaN drops out of the fmax / fmin of the residual maxima and the
+  // ratio test, and a partition left out here is never read again, so a non-finite input could otherwise come back
+  // as a converged solve.  Such a station gets status 2.
   if (tid == 0) {
     int cnt = 0;
+    bool finite = isfinite(x0) && isfinite(derr);  // derr: every Mp and beta
+    for (int k = 0; k < N; ++k) finite = finite && isfinite(a.demand[(size_t)st_idx * N + k]);
     for (int q = 0; q < Q2max; ++q) {
       const bool small = q < P;
       const int p = small ? q : q - P;
@@ -337,6 +342,7 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
       const double th = small ? c.theta_s : c.theta_l;
       const double gq = small ? a.gamma_sm[(size_t)st_idx * P + p] : a.gamma_lm[(size_t)st_idx * P + p];
       const double aq = c.cost_type == 0 ? (th * mp) * (th * mp) : 1.0;
+      finite = finite && isfinite(gq);
       if (th * mp == 0.0 && (gq == 0.0 || aq == 0.0)) continue;
       MQ[cnt] = th * mp;
       AQ[cnt] = aq;
@@ -348,9 +354,11 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
     }
     AV[cnt] = 1.0;
     RED[0] = (double)cnt;
+    RED[1] = finite ? 1.0 : 0.0;
   }
   BI_SYNC();
   const int Q2 = (int)RED[0], QN = Q2 * N, nb = Q2 + 1, np = nb * (nb + 1) / 2;
+  const bool finite_in = RED[1] != 0.0;
   BI_SYNC();
   for (int k = tid; k < N; k += T) {
     DEM[k] = a.demand[(size_t)st_idx * N + k];
@@ -399,6 +407,10 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
   int it = 0, status = 1;
   double mu = 0.0;
   for (;; ++it) {
+    if (!finite_in) {
+      status = 2;
+      break;
+    }
     BI_TIC(0);
     // ---- A. primal quantities and the gradient of the charging cost
     for (int q = tid; q < Q2; q += T) {
