@@ -5,7 +5,8 @@ sm_100a kernel behind ``include/lompc_b200.h``.
 
 Added (not in the reference): ``LoMPC.solve_lompc_batch`` - the same solve for
 a whole batch of (lmbd, lmbd_r, gamma) triples in one kernel launch; the scalar
-``solve_lompc`` is that call with B = 1."""
+``solve_lompc`` is that call with B = 1.  ``LoMPC.solve_lompc_diff`` / ``solve_lompc_vjp`` - the same solve with
+a device-side vector-Jacobian product (chargingstation/autodiff.py)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -202,6 +203,39 @@ class LoMPC:
         if return_info:
             return w, cost, {"status": status, "iters": iters, "kkt_res": kkt}
         return w, cost
+
+    def solve_lompc_diff(self, lmbd, lmbd_r, gamma):
+        """Differentiable ``solve_lompc_batch`` on fp64 CUDA tensors that may require grad (chargingstation/autodiff.py).
+
+        lmbd: [B, 3N] or [3N] (broadcast); lmbd_r: [B], a one-element tensor (broadcast) or a float; gamma: [B].
+        Returns (w[B, N], cost[B]); raises like ``solve_lompc`` on an invalid or unconverged QP (one host sync).
+        Backward: one ``lompc_vjp_dev`` launch; a broadcast input receives the batch sum of the per-QP gradients.
+        A coordinate of w within 1e-9 w_max of a breakpoint counts as fixed; at a weakly active coordinate, where w
+        is not differentiable, the gradient is that of this active set (one of the one-sided derivatives)."""
+        import torch
+
+        from chargingstation.autodiff import LoMPCSolveFunction
+
+        if not torch.is_tensor(lmbd_r):
+            lmbd_r = torch.full((1,), float(lmbd_r), dtype=torch.float64, device=gamma.device)
+        return LoMPCSolveFunction.apply(self, lmbd.contiguous(), lmbd_r.contiguous(), gamma.contiguous())
+
+    def solve_lompc_vjp(self, lmbd, lmbd_r, gamma, w, grad_w=None, grad_cost=None, return_info: bool = False):
+        """Vector-Jacobian product of ``solve_lompc_batch`` outside autograd (``lompc_vjp_dev``, asynchronous on the
+        current torch stream).  ``w`` is the solution at (lmbd, lmbd_r, gamma); grad_w[B, N] / grad_cost[B] are
+        the upstream gradients (None = zero).  Returns per-QP rows (grad_lmbd[B, 3N], grad_lmbd_r[B],
+        grad_gamma[B]) even for broadcast inputs, and with ``return_info`` a dict with the per-QP ``status``
+        (rows with invalid parameters get zero gradients and the solve's status code).  Same active-set
+        convention as ``solve_lompc_diff``."""
+        import torch
+
+        from chargingstation.autodiff import lompc_vjp
+
+        if not torch.is_tensor(lmbd_r):
+            lmbd_r = torch.full((1,), float(lmbd_r), dtype=torch.float64, device=gamma.device)
+        status = torch.empty(gamma.shape, dtype=torch.int32, device=gamma.device) if return_info else None
+        grads = lompc_vjp(self, lmbd, lmbd_r, gamma, w, grad_w, grad_cost, status=status)
+        return (*grads, {"status": status}) if return_info else grads
 
     def wait(self) -> None:
         """Completes a ``solve_lompc_batch(..., wait=False)``; raises like the blocking call."""

@@ -9,6 +9,7 @@
 #include "lompc_common.cuh"
 #include "lompc_solve.cuh"
 #include "lompc_solve_reg.cuh"
+#include "lompc_vjp.cuh"
 #include "lompc_price.cuh"
 #include "lompc_price_fused.cuh"
 #include "lompc_price_warp.cuh"
@@ -223,6 +224,30 @@ inline int64_t warp_kernel_max_batch(int N) {
   return N == 12 ? 4096 : (N == 24 ? 6144 : INT64_MAX);
 }
 
+// Threads per CTA of the one-QP-per-thread kernels with per-stage columns in shared memory ([k*T + t], qp_bytes per
+// QP): the size that keeps most warps resident per SM (shared memory is the limit), capped at 128; small batches use
+// small blocks so that more SMs take part.
+int any_n_cta_width(size_t qp_bytes, int64_t B) {
+  int T = 32;
+  {
+    size_t best = 0;
+    for (int cand = 32; cand <= 128; cand <<= 1) {
+      const size_t per_cta = qp_bytes * cand + 1024;
+      const size_t warps = (size_t)(227 * 1024 / per_cta) * (cand / 32);
+      if (warps >= best && per_cta <= 227 * 1024) {
+        best = warps;
+        T = cand;
+      }
+    }
+  }
+  while (T > 32 && (B + T - 1) / T < 148) T >>= 1;
+  // Horizons whose columns do not fit 32 threads (K1: N > 129 large EV, N > 151 small EV): the largest power of two
+  // that fits.  The kernels have no barrier and their layout is [k*T + t], so any T works; at T = 1 every N <= 4096
+  // fits.  (The throughput of these partial-warp CTAs has not been measured.)
+  while (T > 1 && qp_bytes * T > 227 * 1024) T >>= 1;
+  return T;
+}
+
 template <int NSEG>
 int launch_solve(const lompc_handle* h, const lompc::SolveArgs& a, cudaStream_t stream) {
   const int N = h->cs.N;
@@ -245,25 +270,7 @@ int launch_solve(const lompc_handle* h, const lompc::SolveArgs& a, cudaStream_t 
     if (N == 24) return launch_solve_reg_variant<24, NSEG>(h, a, stream);
     if (N == 12) return launch_solve_reg_variant<12, NSEG>(h, a, stream);
   }
-  // Threads per block: the size that keeps most warps resident per SM (shared memory is the limit: 6-7 vectors of
-  // N doubles per QP), capped at 128; small batches use small blocks so that more SMs take part.
-  int T = 32;
-  {
-    size_t best = 0;
-    for (int cand = 32; cand <= 128; cand <<= 1) {
-      const size_t per_cta = lompc::SmemLayout<NSEG>::bytes(N, cand) + 1024;
-      const size_t warps = (size_t)(227 * 1024 / per_cta) * (cand / 32);
-      if (warps >= best && per_cta <= 227 * 1024) {
-        best = warps;
-        T = cand;
-      }
-    }
-  }
-  while (T > 32 && (a.B + T - 1) / T < 148) T >>= 1;
-  // Horizons whose columns do not fit 32 threads (N > 129 large EV, N > 151 small EV): the largest power of two that
-  // fits.  The kernel has no barrier and its layout is [k*T + t], so any T works; at T = 1 every N <= 4096 fits.
-  // (The throughput of these partial-warp CTAs has not been measured.)
-  while (T > 1 && lompc::SmemLayout<NSEG>::bytes(N, T) > 227 * 1024) T >>= 1;
+  const int T = any_n_cta_width(lompc::SmemLayout<NSEG>::bytes(N, 1), a.B);
   const size_t smem = lompc::SmemLayout<NSEG>::bytes(N, T);
   if (smem > 227 * 1024) return LOMPC_ERR_ARG;
   static std::atomic<uint64_t> configured{0};  // per device ordinal (the attribute is per context)
@@ -274,6 +281,25 @@ int launch_solve(const lompc_handle* h, const lompc::SolveArgs& a, cudaStream_t 
   }
   const int64_t blocks = (a.B + T - 1) / T;
   lompc::lompc_solve_kernel<NSEG><<<(unsigned)blocks, T, smem, stream>>>(h->cs, a);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  CK(cudaGetLastError());
+  return LOMPC_OK;
+}
+
+template <int NSEG>
+int launch_vjp(const lompc_handle* h, const lompc::VjpArgs& a, cudaStream_t stream) {
+  const int N = h->cs.N;
+  const size_t qp_bytes = (size_t)lompc::kVjpArrays * N * sizeof(double);
+  const int T = any_n_cta_width(qp_bytes, a.B);
+  const size_t smem = qp_bytes * T;
+  if (smem > 227 * 1024) return LOMPC_ERR_ARG;
+  static std::atomic<uint64_t> configured{0};  // per device ordinal (the attribute is per context)
+  if (!device_flag_test(configured, h->device)) {
+    CK(cudaFuncSetAttribute(lompc::lompc_vjp_kernel<NSEG>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    device_flag_set(configured, h->device);
+  }
+  const int64_t blocks = (a.B + T - 1) / T;
+  lompc::lompc_vjp_kernel<NSEG><<<(unsigned)blocks, T, smem, stream>>>(h->cs, a);
   g_launches.fetch_add(1, std::memory_order_relaxed);
   CK(cudaGetLastError());
   return LOMPC_OK;
@@ -501,6 +527,33 @@ int lompc_solve_batch_dev(lompc_t* h, int64_t B, const double* lmbd, int64_t lmb
   a.w_init = nullptr;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   return h->cs.large ? launch_solve<4>(h, a, s) : launch_solve<1>(h, a, s);
+}
+
+int lompc_vjp_dev(lompc_t* h, int64_t B, const double* lmbd, int64_t lmbd_stride, const double* lmbd_r,
+                  int64_t lmbd_r_stride, const double* gamma, const double* w, const double* grad_w,
+                  const double* grad_cost, double* grad_lmbd, double* grad_lmbd_r, double* grad_gamma,
+                  int32_t* status, void* stream) {
+  if (!h || B < 0 || !lmbd || !lmbd_r || !gamma || !w) return LOMPC_ERR_ARG;
+  if (lmbd_stride != 0 && lmbd_stride < 3 * (int64_t)h->cs.N) return LOMPC_ERR_ARG;
+  if (lmbd_r_stride != 0 && lmbd_r_stride != 1) return LOMPC_ERR_ARG;
+  if (B == 0) return LOMPC_OK;
+  CK(cudaSetDevice(h->device));
+  lompc::VjpArgs a;
+  a.B = B;
+  a.lmbd = lmbd;
+  a.lmbd_stride = lmbd_stride;
+  a.lmbd_r = lmbd_r;
+  a.lmbd_r_stride = lmbd_r_stride;
+  a.gamma = gamma;
+  a.w = w;
+  a.grad_w = grad_w;
+  a.grad_cost = grad_cost;
+  a.grad_lmbd = grad_lmbd;
+  a.grad_lmbd_r = grad_lmbd_r;
+  a.grad_gamma = grad_gamma;
+  a.status = status;
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  return h->cs.large ? launch_vjp<4>(h, a, s) : launch_vjp<1>(h, a, s);
 }
 
 // Host entry point in two halves: enqueue (copies in, kernel, copies out on the handle's own

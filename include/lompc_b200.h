@@ -89,6 +89,26 @@ int lompc_solve_batch_dev(lompc_t* h, int64_t B, const double* lmbd, int64_t lmb
                           double* w_out, double* cost_out, int32_t* status, int32_t* iters,
                           double* kkt_res, void* stream);
 
+/* Vector-Jacobian product of lompc_solve_batch_dev: for B solved QPs (w[B,N] = their solutions) and upstream
+ * gradients grad_w[B,N] on w and grad_cost[B] on the cost (either may be NULL = zero), writes per QP
+ *   grad_lmbd[B,3N], grad_lmbd_r[B], grad_gamma[B]   (each may be NULL: not computed)
+ * = the gradient of  sum_k grad_w[b,k] w[b,k] + grad_cost[b] cost[b]  with respect to that QP's lmbd row, lmbd_r
+ * and gamma.  lmbd / lmbd_r take the strides of lompc_solve_batch_dev (0 = broadcast); the outputs are per-QP rows
+ * even then (a caller that broadcast sums them over the batch).  One QP per thread, two O(N) sweeps (a Riccati
+ * solve with the upstream gradient as right-hand side, DESIGN.md section 2).  Asynchronous on `stream`, DEVICE
+ * pointers; every N that lompc_create accepts.
+ * Classification: a coordinate of w within 1e-9 w_max of a breakpoint (0, w_max, an interior large-EV pwl
+ * breakpoint) is fixed, the others are free; the w-gradient is that of this active set.  At a weakly active
+ * coordinate (multiplier at an end of its interval) w is not differentiable; the result is then one of the
+ * one-sided derivatives.  The cost gradient (envelope theorem) holds at every point.
+ * A row with a negative or NaN parameter or gamma > y_max gets zero gradients and the solve's status code in the
+ * optional status[B] (LOMPC_ST_NEGATIVE / LOMPC_ST_BAD_GAMMA; LOMPC_ST_OK otherwise).                           */
+int lompc_vjp_dev(lompc_t* h, int64_t B, const double* lmbd, int64_t lmbd_stride,
+                  const double* lmbd_r, int64_t lmbd_r_stride, const double* gamma,
+                  const double* w, const double* grad_w, const double* grad_cost,
+                  double* grad_lmbd, double* grad_lmbd_r, double* grad_gamma,
+                  int32_t* status, void* stream);
+
 /* Same call with HOST buffers: copies in, solves, copies out, synchronises.
  * Returns LOMPC_ERR_GAMMA / LOMPC_ERR_NEGATIVE / LOMPC_ERR_NOT_CONVERGED if
  * any QP reported that status (outputs are still written).                  */
