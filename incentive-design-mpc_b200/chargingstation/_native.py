@@ -46,6 +46,8 @@ SIGNATURES = {
     "lompc_host_wait": (C.c_int, [C.c_void_p]),
     "lompc_vjp_dev": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64] +
                       [C.c_void_p] * 9),
+    "lompc_group_solve_dev": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64] + [C.c_void_p] * 8),
+    "lompc_group_vjp_dev": (C.c_int, [C.c_void_p, C.c_int32, C.c_int64] + [C.c_void_p] * 12),
     "lompc_launch_count": (C.c_int64, []),
     "lompc_set_create": (C.c_int, [C.POINTER(C.c_void_p), C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_void_p)]),
     "lompc_set_destroy": (C.c_int, [C.c_void_p]),

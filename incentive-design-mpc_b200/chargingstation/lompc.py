@@ -6,7 +6,8 @@ sm_100a kernel behind ``include/lompc_b200.h``.
 Added (not in the reference): ``LoMPC.solve_lompc_batch`` - the same solve for
 a whole batch of (lmbd, lmbd_r, gamma) triples in one kernel launch; the scalar
 ``solve_lompc`` is that call with B = 1.  ``LoMPC.solve_lompc_diff`` / ``solve_lompc_vjp`` - the same solve with
-a device-side vector-Jacobian product (chargingstation/autodiff.py)."""
+a device-side vector-Jacobian product (chargingstation/autodiff.py).  ``LoMPC.solve_lompc_groups_diff`` - the
+differentiable solve of groups of EVs that share their group's prices, with the group means."""
 from __future__ import annotations
 
 import ctypes as C
@@ -219,6 +220,27 @@ class LoMPC:
         if not torch.is_tensor(lmbd_r):
             lmbd_r = torch.full((1,), float(lmbd_r), dtype=torch.float64, device=gamma.device)
         return LoMPCSolveFunction.apply(self, lmbd.contiguous(), lmbd_r.contiguous(), gamma.contiguous())
+
+    def solve_lompc_groups_diff(self, group_off, lmbd, lmbd_r, gamma):
+        """Differentiable grouped solve (chargingstation/autodiff.py, ``lompc_group_solve_dev``): EVs sorted by group,
+        group g owns EVs [group_off[g], group_off[g+1]) and every EV of it sees the prices lmbd[g], lmbd_r[g]
+        (the price loop's structure, price_solver.py:196-214).
+
+        group_off: int32 CUDA tensor [G+1] with 0 = off[0] <= off[1] <= ... <= off[G] = B; lmbd: [G, 3N];
+        lmbd_r: [G], a one-element tensor or a float (broadcast to every group); gamma: [B]; fp64 CUDA tensors.
+        Returns (w[B, N], w_avg[G, N]), w_avg the group means (0 for an empty group).  One host sync: ValueError for
+        a malformed group_off, else raises like ``solve_lompc`` on an invalid or unconverged EV.
+        Backward: one ``lompc_group_vjp_dev`` call that writes the [G, 3N] gradient directly, each group's EVs added
+        in EV order (the same bits whatever else is in the batch); a broadcast lmbd_r receives the sum over the
+        groups.  Same active-set convention as ``solve_lompc_diff``."""
+        import torch
+
+        from chargingstation.autodiff import LoMPCGroupSolveFunction
+
+        if not torch.is_tensor(lmbd_r):
+            lmbd_r = torch.full((1,), float(lmbd_r), dtype=torch.float64, device=gamma.device)
+        return LoMPCGroupSolveFunction.apply(self, group_off, lmbd.contiguous(), lmbd_r.contiguous(),
+                                             gamma.contiguous())
 
     def solve_lompc_vjp(self, lmbd, lmbd_r, gamma, w, grad_w=None, grad_cost=None, return_info: bool = False):
         """Vector-Jacobian product of ``solve_lompc_batch`` outside autograd (``lompc_vjp_dev``, asynchronous on the

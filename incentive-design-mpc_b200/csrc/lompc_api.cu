@@ -10,6 +10,7 @@
 #include "lompc_solve.cuh"
 #include "lompc_solve_reg.cuh"
 #include "lompc_vjp.cuh"
+#include "lompc_group_vjp.cuh"
 #include "lompc_price.cuh"
 #include "lompc_price_fused.cuh"
 #include "lompc_price_warp.cuh"
@@ -677,7 +678,8 @@ int ensure_pws(lompc_handle* h, size_t bytes) {
 int launch_group_solve(const lompc_handle* h, int64_t B, const double* lmbd, const double* lmbd_r,
                        const double* gamma, const int32_t* group_of, const int32_t* skip,
                        const double* w_ref, double* w_out, double* cost_out, double* err_out,
-                       double* w0_out, double* price0_out, cudaStream_t s, const double* w_init = nullptr) {
+                       double* w0_out, double* price0_out, cudaStream_t s, const double* w_init = nullptr,
+                       int32_t* status = nullptr) {
   if (B == 0) return LOMPC_OK;
   lompc::SolveArgs a;
   a.B = B;
@@ -688,7 +690,7 @@ int launch_group_solve(const lompc_handle* h, int64_t B, const double* lmbd, con
   a.gamma = gamma;
   a.w_out = w_out;
   a.cost_out = cost_out;
-  a.status = nullptr;
+  a.status = status;
   a.iters = nullptr;
   a.kkt_res = nullptr;
   a.max_iter = h->max_iter;
@@ -727,6 +729,31 @@ int launch_group_step(const lompc_handle* h, const lompc::PriceArgs& p, int it, 
   return LOMPC_OK;
 }
 #define COUNT_LAUNCH() g_launches.fetch_add(1, std::memory_order_relaxed)
+
+// The grouped VJP (lompc_group_vjp.cuh): one EV per thread with the CTA width of launch_vjp, then the group sums.
+template <int NSEG>
+int launch_group_vjp(const lompc_handle* h, const lompc::GroupVjpArgs& a, cudaStream_t stream) {
+  const int N = h->cs.N;
+  const size_t qp_bytes = (size_t)lompc::kVjpArrays * N * sizeof(double);
+  const int T = any_n_cta_width(qp_bytes, a.B);
+  const size_t smem = qp_bytes * T;
+  if (smem > 227 * 1024) return LOMPC_ERR_ARG;
+  static std::atomic<uint64_t> configured{0};  // per device ordinal (the attribute is per context)
+  if (!device_flag_test(configured, h->device)) {
+    CK(cudaFuncSetAttribute(lompc::group_vjp_ev_kernel<NSEG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                            227 * 1024));
+    device_flag_set(configured, h->device);
+  }
+  lompc::group_vjp_ev_kernel<NSEG><<<nblk(a.B, T), T, smem, stream>>>(h->cs, a);
+  COUNT_LAUNCH();
+  CK(cudaGetLastError());
+  if (a.grad_lmbd || a.grad_lmbd_r) {
+    lompc::group_vjp_sum_kernel<<<nblk((int64_t)a.G * N, 128), 128, 0, stream>>>(h->cs, a);
+    COUNT_LAUNCH();
+    CK(cudaGetLastError());
+  }
+  return LOMPC_OK;
+}
 
 }  // namespace
 
@@ -799,6 +826,85 @@ int price_w_err_dev(lompc_t* h, int32_t G, int64_t B, const int32_t* group_off,
   p.w_avg = wa; p.w_err_max = em; p.w_avg_err = w_avg_err ? w_avg_err : t_eavg;
   p.w0_err = w0_err ? w0_err : t_e0; p.skip = skip; p.iters = iters; p.nnqp_status = nst; p.n_active = nact;
   return launch_group_step(h, p, 0, s);
+}
+
+int lompc_group_solve_dev(lompc_t* h, int32_t G, int64_t B, const int32_t* group_off, const double* lmbd,
+                          const double* lmbd_r, const double* gamma, double* w, double* w_avg, int32_t* status,
+                          void* stream) {
+  if (!h || G < 0 || B < 0 || !group_off || (G > 0 && (!lmbd || !lmbd_r || !w_avg)) ||
+      (B > 0 && (!gamma || !w)) || (G == 0 && B > 0))
+    return LOMPC_ERR_ARG;
+  if (G == 0) return LOMPC_OK;
+  CK(cudaSetDevice(h->device));
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int N = h->cs.N;
+  if (B == 0) {
+    CK(cudaMemsetAsync(w_avg, 0, (size_t)G * N * sizeof(double), s));
+    return LOMPC_OK;
+  }
+  Carver sz(nullptr);
+  sz.take<int32_t>(B); sz.take<int32_t>(G); sz.take<int32_t>(G); sz.take<int32_t>(G);
+  int rc = ensure_pws(h, sz.off);
+  if (rc) return rc;
+  Carver cv(h->pws);
+  int32_t* group_of = cv.take<int32_t>(B);
+  int32_t* empty = cv.take<int32_t>(G);
+  int32_t* iters = cv.take<int32_t>(G);
+  int32_t* nst = cv.take<int32_t>(G);
+  lompc::group_of_kernel<<<nblk(B, 256), 256, 0, s>>>(B, G, group_off, group_of);
+  COUNT_LAUNCH();
+  lompc::init_groups_kernel<<<nblk(G, 128), 128, 0, s>>>(G, 1, group_off, empty, iters, nst);
+  COUNT_LAUNCH();
+  rc = launch_group_solve(h, B, lmbd, lmbd_r, gamma, group_of, nullptr, nullptr, w, nullptr, nullptr, nullptr,
+                          nullptr, s, nullptr, status);
+  if (rc) return rc;
+  // the rows of empty groups (skipped by colsum_kernel) stay 0
+  CK(cudaMemsetAsync(w_avg, 0, (size_t)G * N * sizeof(double), s));
+  lompc::colsum_kernel<<<nblk((int64_t)G * N, 128), 128, 0, s>>>(N, G, group_off, empty, w, nullptr, w_avg, nullptr,
+                                                                0);
+  COUNT_LAUNCH();
+  CK(cudaGetLastError());
+  return LOMPC_OK;
+}
+
+int lompc_group_vjp_dev(lompc_t* h, int32_t G, int64_t B, const int32_t* group_off, const double* lmbd,
+                        const double* lmbd_r, const double* gamma, const double* w, const double* grad_w,
+                        const double* grad_w_avg, double* grad_lmbd, double* grad_lmbd_r, double* grad_gamma,
+                        int32_t* status, void* stream) {
+  if (!h || G < 0 || B < 0 || !group_off || (G > 0 && (!lmbd || !lmbd_r)) || (B > 0 && (!gamma || !w)) ||
+      (G == 0 && B > 0))
+    return LOMPC_ERR_ARG;
+  if (G == 0) return LOMPC_OK;
+  CK(cudaSetDevice(h->device));
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  const int N = h->cs.N;
+  if (B == 0) {
+    if (grad_lmbd) CK(cudaMemsetAsync(grad_lmbd, 0, (size_t)G * 3 * N * sizeof(double), s));
+    if (grad_lmbd_r) CK(cudaMemsetAsync(grad_lmbd_r, 0, (size_t)G * sizeof(double), s));
+    return LOMPC_OK;
+  }
+  Carver sz(nullptr);
+  sz.take<double>((size_t)B * N); sz.take<double>(B);
+  int rc = ensure_pws(h, sz.off);
+  if (rc) return rc;
+  Carver cv(h->pws);
+  lompc::GroupVjpArgs a;
+  a.G = G;
+  a.B = B;
+  a.off = group_off;
+  a.lmbd = lmbd;
+  a.lmbd_r = lmbd_r;
+  a.gamma = gamma;
+  a.w = w;
+  a.grad_w = grad_w;
+  a.grad_w_avg = grad_w_avg;
+  a.z = cv.take<double>((size_t)B * N);
+  a.zw = cv.take<double>(B);
+  a.grad_gamma = grad_gamma;
+  a.status = status;
+  a.grad_lmbd = grad_lmbd;
+  a.grad_lmbd_r = grad_lmbd_r;
+  return h->cs.large ? launch_group_vjp<4>(h, a, s) : launch_group_vjp<1>(h, a, s);
 }
 
 int price_step_dev(lompc_t* h, int32_t G, int r, const double* w_ref, const double* w_k,

@@ -49,26 +49,50 @@ struct VjpArgs {
 // (0 on fixed stages) and w_k.
 constexpr int kVjpArrays = 4;
 
-template <int NSEG>
-__global__ void __launch_bounds__(128) lompc_vjp_kernel(const Consts cs, const VjpArgs a) {
-  extern __shared__ double smem[];
-  const int T = blockDim.x;
-  const int t = threadIdx.x;
-  const int N = cs.N;
-  const int64_t b = (int64_t)blockIdx.x * T + t;
-  if (b >= a.B) return;  // no block-level sync below
+// g with off[g] <= b < off[g+1] (binary search; off non-decreasing, off[0] = 0, off[G] > b)
+__device__ __forceinline__ int group_of_ev(int G, const int32_t* __restrict__ off, int64_t b) {
+  int lo = 0, hi = G;
+  while (hi - lo > 1) {
+    const int mid = (lo + hi) >> 1;
+    if ((int64_t)off[mid] <= b) lo = mid; else hi = mid;
+  }
+  return lo;
+}
 
-  double* MM = smem + t;
+// The recursion of QP b, shared by lompc_vjp_kernel (GROUP false, A = VjpArgs) and the grouped VJP's
+// group_vjp_ev_kernel (GROUP true, A = GroupVjpArgs, lompc_group_vjp.cuh).  smem_col: this thread's first column
+// element in the kVjpArrays * N * T doubles of shared memory.  GROUP: QP b takes its group's prices, its upstream is
+// grad_w[b] + grad_w_avg[g] / n_g, and it writes its adjoint z (0 for an invalid EV) and z'w to the workspace
+// instead of gradient rows (no cost term).  (This is the kernel's body as it was written, with the group mode added
+// at compile time: restated with callbacks it needed 8 more registers in the large-EV kernel.)
+template <int NSEG, bool GROUP, class A>
+__device__ __forceinline__ void vjp_qp(const Consts& cs, const A& a, double* smem_col, int T, int64_t b) {
+  const int N = cs.N;
+  double* MM = smem_col;
   double* RR = MM + (size_t)N * T;
   double* IV = RR + (size_t)N * T;
   double* WW = IV + (size_t)N * T;
 
-  const double* lm = a.lmbd + b * a.lmbd_stride;
-  const double lr = a.lmbd_r[b * a.lmbd_r_stride];
+  const double* lm;
+  double lr;
+  const double* ga = nullptr;
+  double n = 0.0;
+  if constexpr (GROUP) {
+    const int g = group_of_ev(a.G, a.off, b);
+    lm = a.lmbd + (int64_t)g * (3 * N);
+    lr = a.lmbd_r[g];
+    ga = a.grad_w_avg ? a.grad_w_avg + (int64_t)g * N : nullptr;
+    n = (double)(a.off[g + 1] - a.off[g]);
+  } else {
+    lm = a.lmbd + b * a.lmbd_stride;
+    lr = a.lmbd_r[b * a.lmbd_r_stride];
+  }
   const double gam = a.gamma[b];
   const double* wr = a.w + b * (int64_t)N;
   const double* gw = a.grad_w ? a.grad_w + b * (int64_t)N : nullptr;
-  const double gc = a.grad_cost ? a.grad_cost[b] : 0.0;
+  double gc = 0.0;
+  if constexpr (!GROUP) gc = a.grad_cost ? a.grad_cost[b] : 0.0;
+  const bool up = GROUP ? (gw || ga) : gw != nullptr;
   const double c = cs.c, wmax = cs.w_max;
   const double band = 1e-9 * wmax;  // K1's binding band (lompc_solve.cuh)
   double blo[NSEG + 1], bhi[NSEG + 1];
@@ -87,9 +111,13 @@ __global__ void __launch_bounds__(128) lompc_vjp_kernel(const Consts cs, const V
     if (!(l1 >= 0.0) || !(l2 >= 0.0) || !(l3 >= 0.0)) st = LOMPC_ST_NEGATIVE;
     const double wk = wr[k];
     WW[k * T] = wk;
-    if (!gw) continue;
+    if (!up) continue;
     const double d = 2.0 * (lr * cs.theta2 + cs.q_scale * l3) + cs.d_base;
-    const double g = gw[k];
+    double g;
+    if constexpr (GROUP)
+      g = (gw ? gw[k] : 0.0) + (ga ? ga[k] / n : 0.0);
+    else
+      g = gw[k];
     bool fixed = wk <= band || wk >= blo[NSEG];
 #pragma unroll
     for (int j = 1; j < NSEG; ++j) fixed |= (wk >= blo[j]) && (wk <= bhi[j]);
@@ -111,26 +139,47 @@ __global__ void __launch_bounds__(128) lompc_vjp_kernel(const Consts cs, const V
   const bool ok = st == LOMPC_ST_OK;
 
   // ---- forward pass: z, then the gradients ---------------------------------------------------------------
-  double* gl = a.grad_lmbd ? a.grad_lmbd + b * (int64_t)(3 * N) : nullptr;
+  double* gl = nullptr;
+  if constexpr (GROUP)
+    gl = a.z + b * (int64_t)N;
+  else
+    gl = a.grad_lmbd ? a.grad_lmbd + b * (int64_t)(3 * N) : nullptr;
   const double th = cs.theta, q = cs.q_scale;
   double sigma = 0.0, s = 0.0, zw = 0.0, zn = 0.0, ww = 0.0, ss = 0.0;
   for (int k = 0; k < N; ++k) {
     const double wk = WW[k * T];
-    const double z = gw ? -fma(MM[k * T], sigma, RR[k * T]) * IV[k * T] : 0.0;
+    const double z = up ? -fma(MM[k * T], sigma, RR[k * T]) * IV[k * T] : 0.0;
     sigma += z;
     s += wk;
     zw = fma(z, wk, zw);
     zn = fma((double)(N - k), z, zn);
     ww = fma(wk, wk, ww);
     ss += s;
-    if (gl) {
+    if constexpr (GROUP) {
+      gl[k] = ok ? z : 0.0;
+    } else if (gl) {
       gl[k] = ok ? fma(gc * th, wk, -th * z) : 0.0;
       gl[N + k] = ok ? fma(gc * th, wmax - wk, th * z) : 0.0;
       gl[2 * N + k] = ok ? q * wk * fma(gc, wk, -2.0 * z) : 0.0;
     }
   }
-  if (a.grad_lmbd_r) a.grad_lmbd_r[b] = ok ? cs.theta2 * fma(gc, ww, -2.0 * zw) : 0.0;
+  if constexpr (GROUP) {
+    a.zw[b] = ok ? zw : 0.0;
+  } else {
+    if (a.grad_lmbd_r) a.grad_lmbd_r[b] = ok ? cs.theta2 * fma(gc, ww, -2.0 * zw) : 0.0;
+  }
   if (a.grad_gamma) a.grad_gamma[b] = ok ? c * fma(-gc, ss, zn) : 0.0;
 }
+
+template <int NSEG>
+__global__ void __launch_bounds__(128) lompc_vjp_kernel(const Consts cs, const VjpArgs a) {
+  extern __shared__ double smem[];
+  const int T = blockDim.x;
+  const int t = threadIdx.x;
+  const int64_t b = (int64_t)blockIdx.x * T + t;
+  if (b >= a.B) return;  // no block-level sync below
+  vjp_qp<NSEG, false>(cs, a, smem + t, T, b);
+}
+
 
 }  // namespace lompc

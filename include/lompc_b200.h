@@ -109,6 +109,32 @@ int lompc_vjp_dev(lompc_t* h, int64_t B, const double* lmbd, int64_t lmbd_stride
                   double* grad_lmbd, double* grad_lmbd_r, double* grad_gamma,
                   int32_t* status, void* stream);
 
+/* Grouped solve: B EVs sorted by group, group g owns EVs [group_off[g], group_off[g+1]) and every EV of it sees the
+ * group's prices lmbd[g] (3N) and lmbd_r[g] (the structure of the price loop, price_solver.py:196-214).  Writes
+ * w[B,N] (each EV's solution: the bits of lompc_solve_batch_dev on the gathered rows) and w_avg[G,N] (the group
+ * means, added in EV order; an empty group's row is 0) and, if status is not NULL, each EV's status (LOMPC_ST_*).
+ * group_off[G+1] must hold 0 = off[0] <= off[1] <= ... <= off[G] = B; it lives in device memory and is not checked
+ * here.  Asynchronous on `stream`, DEVICE pointers; uses the handle's price-loop workspace, so calls on one handle
+ * must not overlap each other or a price loop.  G = 0 or B = 0 launches nothing (w_avg is still zeroed).        */
+int lompc_group_solve_dev(lompc_t* h, int32_t G, int64_t B, const int32_t* group_off, const double* lmbd,
+                          const double* lmbd_r, const double* gamma, double* w, double* w_avg, int32_t* status,
+                          void* stream);
+
+/* Vector-Jacobian product of lompc_group_solve_dev: for the solutions w[B,N] and upstream gradients grad_w[B,N] on w
+ * and grad_w_avg[G,N] on w_avg (either may be NULL = zero), writes
+ *   grad_lmbd[G,3N], grad_lmbd_r[G] (per group) and grad_gamma[B] (per EV)   (each may be NULL: not computed)
+ * = the gradient of  sum grad_w .* w + sum grad_w_avg .* w_avg.  With gw_i = grad_w[i] + grad_w_avg[g] / n_g the
+ * per-EV adjoint z_i is that of lompc_vjp_dev (same classification and conventions), and the group gradients are
+ * its sums over the group's EVs, added in EV order without atomics (DESIGN.md section 2): a group's result has the
+ * same bits whatever else is in the batch.  An EV whose group has a negative or NaN price, or whose gamma is
+ * negative, NaN or > y_max, gets the solve's status code in the optional status[B], zero grad_gamma and contributes
+ * nothing to its group; an empty group gets zeros.  Same workspace, asynchrony and group_off rules as
+ * lompc_group_solve_dev; every N that lompc_create accepts.                                                        */
+int lompc_group_vjp_dev(lompc_t* h, int32_t G, int64_t B, const int32_t* group_off, const double* lmbd,
+                        const double* lmbd_r, const double* gamma, const double* w, const double* grad_w,
+                        const double* grad_w_avg, double* grad_lmbd, double* grad_lmbd_r, double* grad_gamma,
+                        int32_t* status, void* stream);
+
 /* Same call with HOST buffers: copies in, solves, copies out, synchronises.
  * Returns LOMPC_ERR_GAMMA / LOMPC_ERR_NEGATIVE / LOMPC_ERR_NOT_CONVERGED if
  * any QP reported that status (outputs are still written).                  */
