@@ -107,14 +107,22 @@ SIGNATURES = {
     "bimpc_solve_batch_host": (C.c_int, [C.c_void_p, C.c_int32] + [C.c_void_p] * 14),
     # include/fleet_b200.h
     "fleet_partition_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 9),
+    "fleet_partition_sized_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 10),
     "fleet_bimpc_params_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_int32] + [C.c_double] * 5 +
                                [C.c_void_p] * 8 + [C.c_int32, C.c_int32] + [C.c_void_p] * 9),
+    "fleet_bimpc_params_sized_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p] +
+                                     [C.c_double] * 4 + [C.c_void_p] * 8 + [C.c_int32, C.c_int32] + [C.c_void_p] * 9),
     "fleet_wref_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 3),
     "fleet_keep_prices_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32] + [C.c_void_p] * 7),
     "fleet_apply_charge_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_double, C.c_double,
                                          C.c_double, C.c_int64, C.c_int32, C.c_int32] + [C.c_void_p] * 9),
+    "fleet_apply_charge_sized_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_double,
+                                               C.c_double, C.c_double, C.c_int64, C.c_int32, C.c_int32] +
+                                     [C.c_void_p] * 9),
     "fleet_battery_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_double] +
                           [C.c_void_p] * 4 + [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
+    "fleet_battery_sized_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_double, C.c_double, C.c_void_p] +
+                                [C.c_void_p] * 4 + [C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
 }
 
 _lib = None

@@ -24,10 +24,16 @@ conditions; P times fewer sequential loops).
 
 ``rng="numpy"`` draws arrivals on the host from ``np.random.RandomState(seed + s)`` in the
 reference's order (parity with ``ChargingStation`` after ``np.random.seed(seed + s)``);
-``rng="device"`` uses the counter-based generator of ``fleet_apply_charge_dev``."""
+``rng="device"`` uses the counter-based generator of ``fleet_apply_charge_dev``.
+
+Stations may hold different numbers of EVs (``nevs``).  The per-type state stays [S, M] with
+M = max(nevs): station s owns the first nevs[s] slots of its row, and the padding is never read
+or written by the loop (its SoCs are NaN).  The EV-sorted arrays of the price loops hold real EVs
+only, B = sum(nevs)."""
 from __future__ import annotations
 
 import ctypes as C
+import dataclasses
 
 import numpy as np
 
@@ -42,23 +48,39 @@ from chargingstation.settings import (MAX_INITIAL_SOC, MAX_PRICE_SOLVER_ITERATIO
 class ChargingStationFleet:
     def __init__(self, consts: ChargingStationConstants, nstations: int, demand: np.ndarray | None = None,
                  seed: int = 0, rng: str = "device", chain: str = "reference", device: int = 0,
-                 max_price_iter: int = MAX_PRICE_SOLVER_ITERATIONS, tol_type: str | None = None) -> None:
+                 max_price_iter: int = MAX_PRICE_SOLVER_ITERATIONS, tol_type: str | None = None,
+                 nevs: np.ndarray | None = None) -> None:
         """
-        consts:     the station's constants (every station shares them); ``consts.demand`` is
-                    used for all stations unless ``demand`` [S, >= Tf + N_bi + 1] is given.
+        consts:     the stations' constants (every station shares them, except for its number of
+                    EVs); ``consts.demand`` is used for all stations unless ``demand``
+                    [S, >= Tf + N_bi + 1] is given.
         tol_type:   convergence test of the price loops, "avg" or "max" (price_solver.py:121-128);
                     None = PRICE_SOLVER_TOL_TYPE.
+        nevs:       EVs per type of every station, integers >= 1 [S]; None = consts.nEVs_per_EV_type
+                    for every station.  As in the reference, each station's BiMPC is normalised by
+                    its own EV capacity Bcap[s] = (theta_s + theta_l) * nevs[s], so the battery and
+                    grid limits of ``consts.bimpc_consts`` scale with the station's size.  Demand
+                    is absolute (kWh per step): scale each station's row of ``demand`` with its size,
+                    or its BiMPC may have no feasible plan (tools/run_fleet.py::fleet_demand).
         """
         import torch
         assert rng in ("device", "numpy") and chain in ("reference", "partition")
         assert consts.simulation_length >= 1
         assert (consts.horizon_bimpc >= consts.horizon_lompc) and (consts.horizon_lompc >= 1)
         assert consts.nEVs_per_EV_type >= 1 and consts.npartitions >= 1 and nstations >= 1
+        if nevs is None:
+            nevs = np.full(int(nstations), consts.nEVs_per_EV_type, dtype=np.int64)
+        nevs = np.asarray(nevs)
+        assert nevs.shape == (int(nstations),), f"nevs must hold one count per station, got shape {nevs.shape}"
+        assert nevs.dtype.kind in "iu", f"nevs must be integers, got {nevs.dtype}"
+        assert np.all(nevs >= 1), "every station needs at least one EV per type"
+        assert int(nevs.sum(dtype=np.int64)) < 2 ** 31, "sum(nevs) must fit the int32 EV offsets"
+        self.nevs = nevs.astype(np.int64)
         self.torch = torch
         self.dev = torch.device("cuda", device)
         self.device = int(device)
         self.consts = consts
-        self.S, self.M, self.P = int(nstations), consts.nEVs_per_EV_type, consts.npartitions
+        self.S, self.M, self.P = int(nstations), int(self.nevs.max()), consts.npartitions
         self.Tf, self.N_bi, self.N_lo = consts.simulation_length, consts.horizon_bimpc, consts.horizon_lompc
         self.r = 2 * self.N_lo if consts.price_type == "linear" else 3 * self.N_lo
         self.rng_mode, self.chain, self.seed = rng, chain, int(seed)
@@ -75,19 +97,28 @@ class ChargingStationFleet:
         self.bimpc = BiMPC(N_bi, P, consts.bimpc_consts, consts.small_EV_consts, consts.large_EV_consts, device=device)
         self.ev = {"s": consts.small_EV_consts, "l": consts.large_EV_consts}
         self.solver = {k: PriceSolver(N_lo, self.ev[k], consts.price_type, device=device) for k in ("s", "l")}
-        self.Bcap = (self.ev["s"].theta + self.ev["l"].theta) * M
+        # total EV capacity of every station (charging_station.py:101), the BiMPC's normalisation
+        bcap = (self.ev["s"].theta + self.ev["l"].theta) * self.nevs.astype(np.float64)
+        self.Bcap = torch.from_numpy(bcap).to(self.dev)
+        self.B = int(self.nevs.sum())  # real EVs per type
+        self._nevs = torch.from_numpy(self.nevs.astype(np.int32)).to(self.dev)
         f64, i32 = torch.float64, torch.int32
         z = lambda *shape, dtype=f64: torch.zeros(shape, dtype=dtype, device=self.dev)  # noqa: E731
         # ---- state
         if rng == "numpy":
             self._rs = [np.random.RandomState(self.seed + s) for s in range(S)]
-            y0 = {"s": np.empty((S, M)), "l": np.empty((S, M))}
+            y0 = {"s": np.full((S, M), np.nan), "l": np.full((S, M), np.nan)}
             for s in range(S):  # charging_station.py:95-100: small first, then large
+                n = int(self.nevs[s])
                 for k in ("s", "l"):
-                    y0[k][s] = MIN_INITIAL_SOC + (MAX_INITIAL_SOC - MIN_INITIAL_SOC) * self._rs[s].random_sample((M,))
+                    y0[k][s, :n] = MIN_INITIAL_SOC + (MAX_INITIAL_SOC - MIN_INITIAL_SOC) * \
+                        self._rs[s].random_sample((n,))
         else:
             g = np.random.default_rng(self.seed)
             y0 = {k: MIN_INITIAL_SOC + (MAX_INITIAL_SOC - MIN_INITIAL_SOC) * g.random((S, M)) for k in ("s", "l")}
+            pad = np.arange(M)[None, :] >= self.nevs[:, None]  # slots that hold no EV
+            for k in ("s", "l"):
+                y0[k][pad] = np.nan
         self.y = {k: torch.from_numpy(y0[k]).to(self.dev) for k in ("s", "l")}
         self.idx = {k: z(S, M, dtype=i32) for k in ("s", "l")}
         self.x = z(S)
@@ -99,7 +130,7 @@ class ChargingStationFleet:
         self.edges = {k: torch.from_numpy(partition_edges(MIN_INITIAL_SOC, self.ev[k].y_max, P)).to(self.dev)
                       for k in ("s", "l")}
         # ---- per-step work buffers
-        G, B = P * S, S * M
+        G, B = P * S, self.B
         self.w = {}
         for k in ("s", "l"):
             self.w[k] = dict(counts=z(G, dtype=i32), off=z(G + 1, dtype=i32), reb=z(P, S + 1, dtype=i32),
@@ -152,7 +183,7 @@ class ChargingStationFleet:
     def step(self) -> None:
         torch, lib, st = self.torch, self._lib, self._stream()
         S, M, P, N_lo, N_bi, t = self.S, self.M, self.P, self.N_lo, self.N_bi, self.t
-        G, B = P * S, S * M
+        G, B = P * S, self.B
         lmbd_r = 0.0  # charging_station.py:162
         tol_max = tol_type_max(self.tol_type, PRICE_SOLVER_TOL_TYPE)
         marks = []
@@ -167,17 +198,18 @@ class ChargingStationFleet:
         # ---- partitions, group statistics
         for k in ("s", "l"):
             w, h = self.w[k], self.solver[k]._h
-            self._ck(lib.fleet_partition_dev(self.device, S, M, P, self.edges[k].data_ptr(), self.y[k].data_ptr(),
-                                             self.idx[k].data_ptr(), w["counts"].data_ptr(), w["off"].data_ptr(),
-                                             w["reb"].data_ptr(), w["ysort"].data_ptr(), w["perm"].data_ptr(), st))
+            self._ck(lib.fleet_partition_sized_dev(
+                self.device, S, M, P, self._nevs.data_ptr(), self.edges[k].data_ptr(), self.y[k].data_ptr(),
+                self.idx[k].data_ptr(), w["counts"].data_ptr(), w["off"].data_ptr(), w["reb"].data_ptr(),
+                w["ysort"].data_ptr(), w["perm"].data_ptr(), st))
             self._ck(lib.price_group_stats_dev(h, G, B, w["off"].data_ptr(), w["ysort"].data_ptr(),
                                                w["gamma"].data_ptr(), w["y0_rng"].data_ptr(),
                                                w["gamma_sc"].data_ptr(), w["gamma_sm"].data_ptr(), st))
         mark("partition+stats")
         # ---- upper level
         ws, wl, bi = self.w["s"], self.w["l"], self.bi
-        self._ck(lib.fleet_bimpc_params_dev(
-            self.device, S, P, N_bi, N_lo, float(self.Bcap), float(self.solver["s"].eps_tol), lmbd_r,
+        self._ck(lib.fleet_bimpc_params_sized_dev(
+            self.device, S, P, N_bi, N_lo, self.Bcap.data_ptr(), float(self.solver["s"].eps_tol), lmbd_r,
             float(self.ev["s"].delta), float(self.ev["l"].delta), ws["counts"].data_ptr(), wl["counts"].data_ptr(),
             ws["y0_rng"].data_ptr(), wl["y0_rng"].data_ptr(), ws["gamma_sm"].data_ptr(), wl["gamma_sm"].data_ptr(),
             self.x.data_ptr(), self.demand.data_ptr(), self.profile_len, t, bi["Mp_s"].data_ptr(),
@@ -274,17 +306,17 @@ class ChargingStationFleet:
         for ti, k in enumerate(("s", "l")):
             w = self.w[k]
             seed = self.seed if self.rng_mode == "device" else -1
-            self._ck(lib.fleet_apply_charge_dev(
-                self.device, S, M, P, float(MIN_FULL_CHARGE_FRACTION * self.ev[k].y_max), float(MIN_INITIAL_SOC),
-                float(MAX_INITIAL_SOC), seed, ti, t, w["off"].data_ptr(), w["perm"].data_ptr(), w["w0"].data_ptr(),
-                self.y[k].data_ptr(), w["mask"].data_ptr(), w["w_sum"].data_ptr(), w["w_mean"].data_ptr(),
-                self.ncharged[k].data_ptr(), st))
+            self._ck(lib.fleet_apply_charge_sized_dev(
+                self.device, S, M, P, self._nevs.data_ptr(), float(MIN_FULL_CHARGE_FRACTION * self.ev[k].y_max),
+                float(MIN_INITIAL_SOC), float(MAX_INITIAL_SOC), seed, ti, t, w["off"].data_ptr(),
+                w["perm"].data_ptr(), w["w0"].data_ptr(), self.y[k].data_ptr(), w["mask"].data_ptr(),
+                w["w_sum"].data_ptr(), w["w_mean"].data_ptr(), self.ncharged[k].data_ptr(), st))
         if self.rng_mode == "numpy":
             self._host_arrivals()
-        self._ck(lib.fleet_battery_dev(self.device, S, N_bi, float(self.ev["s"].theta), float(self.ev["l"].theta),
-                                       float(self.Bcap), bi["u_g"].data_ptr(), ws["w_sum"].data_ptr(),
-                                       wl["w_sum"].data_ptr(), self.demand.data_ptr(), self.profile_len, t,
-                                       self.x.data_ptr(), st))
+        self._ck(lib.fleet_battery_sized_dev(self.device, S, N_bi, float(self.ev["s"].theta),
+                                             float(self.ev["l"].theta), self.Bcap.data_ptr(), bi["u_g"].data_ptr(),
+                                             ws["w_sum"].data_ptr(), wl["w_sum"].data_ptr(), self.demand.data_ptr(),
+                                             self.profile_len, t, self.x.data_ptr(), st))
         for k in ("s", "l"):
             w = self.w[k]
             L[f"w_{k}"][t].copy_(w["w_mean"].view(P, S))
@@ -308,10 +340,11 @@ class ChargingStationFleet:
         masks = {k: self.w[k]["mask"].cpu().numpy().astype(bool) for k in ("s", "l")}
         ys = {k: self.y[k].cpu().numpy() for k in ("s", "l")}
         for s in range(self.S):
+            m = int(self.nevs[s])  # the padding of a row is no EV
             for k in ("s", "l"):
-                n = int(masks[k][s].sum())
-                ys[k][s, masks[k][s]] = MIN_INITIAL_SOC + (MAX_INITIAL_SOC - MIN_INITIAL_SOC) * \
-                    self._rs[s].random_sample((n,))
+                leave = masks[k][s, :m]
+                ys[k][s, :m][leave] = MIN_INITIAL_SOC + (MAX_INITIAL_SOC - MIN_INITIAL_SOC) * \
+                    self._rs[s].random_sample((int(leave.sum()),))
         for k in ("s", "l"):
             self.y[k].copy_(torch.from_numpy(ys[k]))
 
@@ -322,11 +355,15 @@ class ChargingStationFleet:
 
     # ------------------------------------------------------------------ logs in the reference schema
     def station_logs(self, s: int) -> dict:
-        """``ChargingStation.logs`` of station s (charging_station.py:118-149)."""
+        """``ChargingStation.logs`` of station s (charging_station.py:118-149); its constants carry
+        the station's own number of EVs."""
         L = {k: v[:, ..., s].cpu().numpy() if v.dim() == 3 else v[:, s].cpu().numpy() for k, v in self.log.items()}
         T = lambda a: np.ascontiguousarray(a.T)  # noqa: E731  [Tf, P] -> [P, Tf]
+        consts = self.consts
+        if int(self.nevs[s]) != consts.nEVs_per_EV_type:
+            consts = dataclasses.replace(consts, nEVs_per_EV_type=int(self.nevs[s]))
         return {
-            "constants": self.consts,
+            "constants": consts,
             "inputs": {"w_s": T(L["w_s"]), "w_l": T(L["w_l"]), "w_hat_s": T(L["w_hat_s"]), "w_hat_l": T(L["w_hat_l"]),
                        "u_g": L["u_g"]},
             "states": {"x": L["x"]},

@@ -10,6 +10,14 @@
  * so that "partition p of every station" is one contiguous slice of groups and of EVs
  * (the reference solves the partitions of an EV type one after the other with a shared
  * warm start, charging_station.py:273-304).
+ *
+ * Stations of different sizes.  The *_sized_dev entry points take nevs[S] (device, 1 <=
+ * nevs[s] <= M; values outside [0, M] are clamped to it) and/or Bcap[S] (device, > 0):
+ * station s owns the first nevs[s] slots of its row of M, and the padding slots of y, idx
+ * and replace_mask are neither read nor written.  The EV-sorted arrays (y_sorted, perm and
+ * what the price loops build on them) hold real EVs only, so off[P*S] = sum(nevs).  The
+ * uniform entry points are the same kernels with nevs[s] = M and Bcap[s] = Bcap for every
+ * station.
  */
 #ifndef FLEET_B200_H
 #define FLEET_B200_H
@@ -31,6 +39,11 @@ extern "C" {
 int fleet_partition_dev(int device, int32_t S, int32_t M, int32_t P, const double* edges, const double* y,
                         int32_t* idx, int32_t* counts, int32_t* off, int32_t* off_rebased,
                         double* y_sorted, int32_t* perm, void* stream);
+/* The same for stations of nevs[s] EVs: only slots j < nevs[s] of a row are assigned and
+ * sorted; counts, off, off_rebased, y_sorted and perm[sum(nevs)] cover real EVs only.      */
+int fleet_partition_sized_dev(int device, int32_t S, int32_t M, int32_t P, const int32_t* nevs, const double* edges,
+                              const double* y, int32_t* idx, int32_t* counts, int32_t* off, int32_t* off_rebased,
+                              double* y_sorted, int32_t* perm, void* stream);
 
 /* BiMPCParameters of every station (charging_station.py:187-220): Mp = counts / Bcap,
  * beta = the w0 bound of PriceSolver.get_robustness_bounds (price_solver.py:182-186) from
@@ -43,6 +56,14 @@ int fleet_bimpc_params_dev(int device, int32_t S, int32_t P, int32_t N_bi, int32
                            const double* x, const double* demand_profile, int32_t profile_len, int32_t t,
                            double* Mp_s, double* Mp_l, double* beta_s, double* beta_l, double* gamma_s,
                            double* gamma_l, double* x0, double* demand, void* stream);
+/* The same with each station's own capacity: Mp = counts / Bcap[s], demand = profile / Bcap[s]. */
+int fleet_bimpc_params_sized_dev(int device, int32_t S, int32_t P, int32_t N_bi, int32_t N_lo, const double* Bcap,
+                                 double eps_tol, double lmbd_r, double delta_s, double delta_l,
+                                 const int32_t* counts_s, const int32_t* counts_l, const double* y0_rng_s,
+                                 const double* y0_rng_l, const double* gamma_sm_s, const double* gamma_sm_l,
+                                 const double* x, const double* demand_profile, int32_t profile_len, int32_t t,
+                                 double* Mp_s, double* Mp_l, double* beta_s, double* beta_l, double* gamma_s,
+                                 double* gamma_l, double* x0, double* demand, void* stream);
 
 /* w_ref of every group = the first N_lo steps of the BiMPC plan (charging_station.py:269):
  * w_ref[(p*S+s), k] = w_hat[s, p, k].                                                      */
@@ -67,6 +88,13 @@ int fleet_apply_charge_dev(int device, int32_t S, int32_t M, int32_t P, double f
                            double y0_max, int64_t rng_seed, int32_t ev_type, int32_t t, const int32_t* off,
                            const int32_t* perm, const double* w0_sorted, double* y, int32_t* replace_mask,
                            double* w_sum, double* w_mean, int32_t* ncharged, void* stream);
+/* The same for stations of nevs[s] EVs: departures, arrivals and replace_mask cover slots
+ * j < nevs[s] only (the generator key keeps the EV's slot in its station).                 */
+int fleet_apply_charge_sized_dev(int device, int32_t S, int32_t M, int32_t P, const int32_t* nevs, double full_level,
+                                 double y0_min, double y0_max, int64_t rng_seed, int32_t ev_type, int32_t t,
+                                 const int32_t* off, const int32_t* perm, const double* w0_sorted, double* y,
+                                 int32_t* replace_mask, double* w_sum, double* w_mean, int32_t* ncharged,
+                                 void* stream);
 
 /* Battery update (charging_station.py:353-365, ADD_RESIDUAL_CHARGE_TO_BATTERY = False):
  * x[s] += u_g[s,0] + (-theta_s w_sum_s[s] - theta_l w_sum_l[s] - profile[s,t]) / Bcap.      */
@@ -74,6 +102,10 @@ int fleet_battery_dev(int device, int32_t S, int32_t N_bi, double theta_s, doubl
                       const double* u_g, const double* w_sum_s, const double* w_sum_l,
                       const double* demand_profile, int32_t profile_len, int32_t t, double* x,
                       void* stream);
+/* The same with each station's own capacity: ... / Bcap[s].                               */
+int fleet_battery_sized_dev(int device, int32_t S, int32_t N_bi, double theta_s, double theta_l, const double* Bcap,
+                            const double* u_g, const double* w_sum_s, const double* w_sum_l,
+                            const double* demand_profile, int32_t profile_len, int32_t t, double* x, void* stream);
 
 #ifdef __cplusplus
 }

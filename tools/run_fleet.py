@@ -3,6 +3,7 @@
 Prints one JSON line: per-step latency (CUDA events), p50/p95, price-loop iterations.
 
     python tools/run_fleet.py --stations 4096 --steps 96 --chain reference
+    python tools/run_fleet.py --stations 4096 --steps 16 --evs-min 100 --evs-max 900 --profile   # mixed sizes
 """
 import argparse
 import json
@@ -46,11 +47,34 @@ def fleet_demand(consts, S, steps, N_bi, seed=4):
     return out
 
 
+def station_sizes(S, lo, hi, seed=5):
+    """EVs per type of every station, uniform on {lo..hi} from a fixed seed."""
+    return np.random.default_rng(seed).integers(lo, hi + 1, S)
+
+
+def card():
+    """Name and power limit of cuda:0 (the power limit is read, never set)."""
+    import subprocess
+
+    import torch
+    out = {"gpu": torch.cuda.get_device_name(0)}
+    try:
+        q = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=power.limit", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=30)
+        out["power_limit"] = q.stdout.strip() or "unknown"
+    except (OSError, subprocess.SubprocessError):
+        out["power_limit"] = "unknown"
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--stations", type=int, default=64)
     ap.add_argument("--steps", type=int, default=8)
     ap.add_argument("--evs", type=int, default=500)
+    ap.add_argument("--evs-min", type=int, default=None,
+                    help="with --evs-max: station sizes uniform on {min..max}, demand scaled by size / 500")
+    ap.add_argument("--evs-max", type=int, default=None)
     ap.add_argument("--partitions", type=int, default=12)
     ap.add_argument("--n-lo", type=int, default=24)
     ap.add_argument("--n-bi", type=int, default=24)
@@ -61,10 +85,17 @@ def main():
     args = ap.parse_args()
     import torch
     from chargingstation.fleet import ChargingStationFleet
-    consts = fleet_consts(args.steps, args.n_lo, args.n_bi, args.evs, args.partitions)
-    demand = fleet_demand(consts, args.stations, args.steps, args.n_bi)
+    nevs = None
+    if args.evs_min is not None or args.evs_max is not None:
+        assert args.evs_min is not None and args.evs_max is not None and 1 <= args.evs_min <= args.evs_max
+        nevs = station_sizes(args.stations, args.evs_min, args.evs_max)
+        consts = fleet_consts(args.steps, args.n_lo, args.n_bi, 500, args.partitions)
+        demand = fleet_demand(consts, args.stations, args.steps, args.n_bi) * (nevs[:, None] / 500)
+    else:
+        consts = fleet_consts(args.steps, args.n_lo, args.n_bi, args.evs, args.partitions)
+        demand = fleet_demand(consts, args.stations, args.steps, args.n_bi)
     fleet = ChargingStationFleet(consts, args.stations, demand=demand, seed=4, rng="device", chain=args.chain,
-                                 max_price_iter=args.max_price_iter)
+                                 max_price_iter=args.max_price_iter, nevs=nevs)
     fleet.profile = args.profile
     for k in ("s", "l"):
         fleet.solver[k].set_loop_mode(args.loop_mode)
@@ -82,8 +113,10 @@ def main():
         wall.append((time.perf_counter() - t0) * 1e3)
     ms = np.array([a.elapsed_time(b) for a, b in zip(ev0, ev1)])
     log = fleet.log
-    out = {"loop_mode": args.loop_mode, "pivot_overflows": [fleet.solver[k].last_pivot_overflows() for k in ("s", "l")],
-           "config": f"{args.stations} stations x ({args.evs}+{args.evs}) EVs, P={args.partitions}, N_lo={args.n_lo}, "
+    sizes = (f"{args.evs}+{args.evs}" if nevs is None else f"U{{{args.evs_min}..{args.evs_max}}} per type")
+    out = {**card(), "loop_mode": args.loop_mode,
+           "pivot_overflows": [fleet.solver[k].last_pivot_overflows() for k in ("s", "l")],
+           "config": f"{args.stations} stations x ({sizes}) EVs, P={args.partitions}, N_lo={args.n_lo}, "
                      f"N_bi={args.n_bi}, {args.steps} closed-loop steps, chain={args.chain}",
            "step_ms_p50": float(np.median(ms)), "step_ms_p95": float(np.percentile(ms, 95)),
            "step_ms_first": float(ms[0]), "step_ms_mean": float(ms.mean()), "wall_ms_p50": float(np.median(wall)),
@@ -93,8 +126,12 @@ def main():
            "price_loop_qp_solves": int(fleet.qp_solves), "qp_solves_per_s": fleet.qp_solves / (ms.sum() * 1e-3),
            "cycles_lompc_passes": fleet.cycles[0], "cycles_price_steps": fleet.cycles[1],
            "k1_iters_per_solve": fleet.cycles[2] / max(1, fleet.qp_solves), "warp_passes_without_k1_iteration": fleet.cycles[3] / max(1, fleet.cycles[4])}
+    out["evs_per_type"] = {"total": int(fleet.B), "mean": float(fleet.nevs.mean()), "min": int(fleet.nevs.min()),
+                           "p50": float(np.median(fleet.nevs)), "p95": float(np.percentile(fleet.nevs, 95)),
+                           "max": int(fleet.nevs.max())}
     if args.profile:
         out["phase_ms_median"] = {k: float(np.median([d[k] for d in fleet.phase_ms])) for k in fleet.phase_ms[0]}
+        out["phase_ms_p95"] = {k: float(np.percentile([d[k] for d in fleet.phase_ms], 95)) for k in fleet.phase_ms[0]}
     for k in ("s", "l"):
         ni = log[f"niter_{k}"].cpu().numpy()
         mp = log[f"Mp_{k}"].cpu().numpy()
