@@ -105,6 +105,9 @@ SIGNATURES = {
     "bimpc_set_options": (C.c_int, [C.c_void_p, C.c_int, C.c_double]),
     "bimpc_solve_batch_dev": (C.c_int, [C.c_void_p, C.c_int32] + [C.c_void_p] * 15),
     "bimpc_solve_batch_host": (C.c_int, [C.c_void_p, C.c_int32] + [C.c_void_p] * 14),
+    "bimpc_stage_weights": (C.c_int, [C.c_int, C.c_int, C.c_double, C.c_void_p]),
+    "bimpc_solve_batch_consts_dev": (C.c_int, [C.c_void_p, C.c_int32] + [C.c_void_p] * 22),
+    "bimpc_solve_batch_consts_host": (C.c_int, [C.c_void_p, C.c_int32] + [C.c_void_p] * 21),
     # include/fleet_b200.h
     "fleet_partition_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 9),
     "fleet_partition_sized_dev": (C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_int32] + [C.c_void_p] * 10),

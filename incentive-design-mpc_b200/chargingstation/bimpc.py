@@ -5,7 +5,8 @@ and return shapes (bimpc.py:12-295).  The convex program cvxpy hands to CLARABEL
 ``include/bimpc_b200.h`` (``csrc/bimpc_solve.cuh``): one station per CTA, block-tridiagonal
 Cholesky over the horizon.  There is no CPU fallback.
 
-Added (not in the reference): ``BiMPC.solve_bimpc_batch`` - S stations in one launch."""
+Added (not in the reference): ``BiMPC.solve_bimpc_batch`` - S stations in one launch, optionally each with
+its own ``BiMPCConstants``."""
 from __future__ import annotations
 
 import ctypes as C
@@ -68,6 +69,45 @@ class BiMPCParameters:
     demand: np.ndarray
 
 
+# the scalar fields of BiMPCConstants that may differ from station to station (with the cost type and exp_rate)
+SCALAR_FIELDS = ("delta", "c_g", "u_g_max", "u_b_max", "x_max")
+
+
+def check_constants(consts_bi: BiMPCConstants, station: int | None = None) -> None:
+    """The asserts of bimpc.py:79-84 (AssertionError) and the cost-type check of bimpc.py:231
+    (NotImplementedError).  ``station``: the index the message names."""
+    where = "" if station is None else f"station {station}: "
+    for f in SCALAR_FIELDS:
+        v = getattr(consts_bi, f)
+        assert v >= 0, f"{where}BiMPCConstants.{f} must be >= 0, got {v}"
+    assert consts_bi.exp_rate >= 1, f"{where}BiMPCConstants.exp_rate must be >= 1, got {consts_bi.exp_rate}"
+    if not isinstance(consts_bi.charging_cost_type, BiMPCChargingCostType):
+        raise NotImplementedError(f"{where}unknown charging cost type {consts_bi.charging_cost_type!r}")  # bimpc.py:231
+
+
+def station_constants(consts, S: int) -> dict:
+    """Checks one ``BiMPCConstants`` per station (``check_constants``, naming the station) and returns them as arrays:
+    delta, c_g, u_g_max, u_b_max, x_max, exp_rate (float64 [S]), cost_type (int32 [S]) and the list itself
+    ("consts")."""
+    assert not isinstance(consts, BiMPCConstants), f"expected one BiMPCConstants per station ({S}), got one in all"
+    consts = list(consts)
+    assert len(consts) == S, f"expected one BiMPCConstants per station ({S}), got {len(consts)}"
+    for s, c in enumerate(consts):
+        check_constants(c, s)
+    out = {f: np.array([float(getattr(c, f)) for c in consts], dtype=np.float64) for f in SCALAR_FIELDS + ("exp_rate",)}
+    out["cost_type"] = np.array([c.charging_cost_type.value for c in consts], dtype=np.int32)
+    out["consts"] = consts
+    return out
+
+
+def stage_weights(lib, N: int, cost_type: int, exp_rate: float) -> np.ndarray:
+    """The [N] stage weights of the charging cost (bimpc.py:255-257) as the library builds them for a handle
+    (``bimpc_stage_weights``): a per-station row has the bits of the handle's."""
+    om = np.empty(N)
+    _native.raise_for(lib.bimpc_stage_weights(int(N), int(cost_type), float(exp_rate), om.ctypes.data_as(C.c_void_p)))
+    return om
+
+
 class BiMPC:
     def __init__(self, N: int, P: int, consts_bi: BiMPCConstants, consts_s: LoMPCConstants,
                  consts_l: LoMPCConstants, device: int = 0) -> None:
@@ -79,15 +119,7 @@ class BiMPC:
             consts_s:           LoMPC constants for small EVs.
             consts_l:           LoMPC constants for large EVs.
         """
-        # bimpc.py:79-84
-        assert consts_bi.delta >= 0
-        assert consts_bi.c_g >= 0
-        assert consts_bi.u_g_max >= 0
-        assert consts_bi.u_b_max >= 0
-        assert consts_bi.x_max >= 0
-        assert consts_bi.exp_rate >= 1
-        if not isinstance(consts_bi.charging_cost_type, BiMPCChargingCostType):
-            raise NotImplementedError  # bimpc.py:231
+        check_constants(consts_bi)  # bimpc.py:79-84, 231
         self.N, self.P = N, P
         self.delta = consts_bi.delta
         self.c_g = consts_bi.c_g
@@ -151,13 +183,19 @@ class BiMPC:
             return None, None, None
         return ws[0], wl[0], ug[0]
 
-    def solve_bimpc_batch(self, Mp_s, Mp_l, beta_s, beta_l, gamma_sm, gamma_lm, x0, demand):
+    def solve_bimpc_batch(self, Mp_s, Mp_l, beta_s, beta_l, gamma_sm, gamma_lm, x0, demand, consts=None):
         """``solve_bimpc`` for S stations: every argument has a leading station axis
         ([S,P] / [S] / [S,N]).  Returns (w_hat_s [S,P,N], w_hat_l [S,P,N], u_g [S,N], info)
-        with info = {status, iters, objective} arrays of length S."""
+        with info = {status, iters, objective} arrays of length S.
+
+        consts: None, or one ``BiMPCConstants`` per station (same units as the constructor's).  Station s
+        then solves with its own delta, c_g, limits, cost type and exp_rate, with the bits a BiMPC created
+        with ``consts[s]`` gives it; N, P and the EV constants stay this object's.  Each is checked like
+        the constructor's constants before any device work."""
         P, N = self.P, self.N
         ins = [np.ascontiguousarray(v, dtype=np.float64) for v in (Mp_s, Mp_l, beta_s, beta_l, gamma_sm, gamma_lm)]
         S = ins[0].shape[0]
+        sc = None if consts is None else station_constants(consts, S)
         for v in ins:
             assert v.shape == (S, P)
             if np.any(v < 0):  # nonneg cv.Parameters, bimpc.py:122-140
@@ -174,8 +212,13 @@ class BiMPC:
         it = np.empty(S, dtype=np.int32)
         obj = np.empty(S)
         p = lambda a: a.ctypes.data_as(C.c_void_p)  # noqa: E731
-        rc = self._lib.bimpc_solve_batch_host(self._h, S, *[p(v) for v in ins], p(x0), p(demand), p(ws), p(wl),
-                                              p(ug), p(st), p(it), p(obj))
+        if sc is None:
+            rc = self._lib.bimpc_solve_batch_host(self._h, S, *[p(v) for v in ins], p(x0), p(demand), p(ws), p(wl),
+                                                  p(ug), p(st), p(it), p(obj))
+        else:
+            rc = self._lib.bimpc_solve_batch_consts_host(
+                self._h, S, *[p(sc[f]) for f in SCALAR_FIELDS + ("cost_type", "exp_rate")], *[p(v) for v in ins], p(x0),
+                p(demand), p(ws), p(wl), p(ug), p(st), p(it), p(obj))
         if rc != _native.ERR_NOT_CONVERGED:
             _native.raise_for(rc)
         # a failed solve yields None in the reference (.value of an unsolved variable, bimpc.py:288-291); the batch

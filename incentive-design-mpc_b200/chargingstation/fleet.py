@@ -29,7 +29,11 @@ reference's order (parity with ``ChargingStation`` after ``np.random.seed(seed +
 Stations may hold different numbers of EVs (``nevs``).  The per-type state stays [S, M] with
 M = max(nevs): station s owns the first nevs[s] slots of its row, and the padding is never read
 or written by the loop (its SoCs are NaN).  The EV-sorted arrays of the price loops hold real EVs
-only, B = sum(nevs)."""
+only, B = sum(nevs).
+
+Stations may also have their own BiMPC constants (``bimpc_consts``): battery capacity and rate, grid
+limit, generation cost, charging-cost weight, cost type and exp_rate.  The BiMPC of every station then
+runs in the same one launch per step (``bimpc_solve_batch_consts_dev``)."""
 from __future__ import annotations
 
 import ctypes as C
@@ -38,7 +42,7 @@ import dataclasses
 import numpy as np
 
 from chargingstation import _native
-from chargingstation.bimpc import BiMPC
+from chargingstation.bimpc import SCALAR_FIELDS, BiMPC, stage_weights, station_constants
 from chargingstation.charging_station import ChargingStationConstants, partition_edges
 from chargingstation.price_solver import PriceSolver, tol_type_max
 from chargingstation.settings import (MAX_INITIAL_SOC, MAX_PRICE_SOLVER_ITERATIONS, MIN_FULL_CHARGE_FRACTION,
@@ -49,10 +53,10 @@ class ChargingStationFleet:
     def __init__(self, consts: ChargingStationConstants, nstations: int, demand: np.ndarray | None = None,
                  seed: int = 0, rng: str = "device", chain: str = "reference", device: int = 0,
                  max_price_iter: int = MAX_PRICE_SOLVER_ITERATIONS, tol_type: str | None = None,
-                 nevs: np.ndarray | None = None) -> None:
+                 nevs: np.ndarray | None = None, bimpc_consts=None) -> None:
         """
         consts:     the stations' constants (every station shares them, except for its number of
-                    EVs); ``consts.demand`` is used for all stations unless ``demand``
+                    EVs and its BiMPC constants); ``consts.demand`` is used for all stations unless ``demand``
                     [S, >= Tf + N_bi + 1] is given.
         tol_type:   convergence test of the price loops, "avg" or "max" (price_solver.py:121-128);
                     None = PRICE_SOLVER_TOL_TYPE.
@@ -62,6 +66,10 @@ class ChargingStationFleet:
                     grid limits of ``consts.bimpc_consts`` scale with the station's size.  Demand
                     is absolute (kWh per step): scale each station's row of ``demand`` with its size,
                     or its BiMPC may have no feasible plan (tools/run_fleet.py::fleet_demand).
+        bimpc_consts: one ``BiMPCConstants`` per station [S]; None = ``consts.bimpc_consts`` for every
+                    station.  Each is checked like ``BiMPC``'s constants, in the units of
+                    ``consts.bimpc_consts`` (normalised by the station's own Bcap[s]).  Station s then
+                    plans with its own battery, grid limit, costs, cost type and exp_rate.
         """
         import torch
         assert rng in ("device", "numpy") and chain in ("reference", "partition")
@@ -76,6 +84,9 @@ class ChargingStationFleet:
         assert np.all(nevs >= 1), "every station needs at least one EV per type"
         assert int(nevs.sum(dtype=np.int64)) < 2 ** 31, "sum(nevs) must fit the int32 EV offsets"
         self.nevs = nevs.astype(np.int64)
+        # per-station BiMPC constants: checked here, before any device work
+        sc = None if bimpc_consts is None else station_constants(bimpc_consts, int(nstations))
+        self.bimpc_consts = [consts.bimpc_consts] * int(nstations) if sc is None else sc["consts"]
         self.torch = torch
         self.dev = torch.device("cuda", device)
         self.device = int(device)
@@ -95,6 +106,13 @@ class ChargingStationFleet:
         self.profile_len = demand.shape[1]
         self._lib = _native.load()
         self.bimpc = BiMPC(N_bi, P, consts.bimpc_consts, consts.small_EV_consts, consts.large_EV_consts, device=device)
+        # device copies of the per-station constants, with each station's stage weights [S, N_bi] built like the
+        # handle's (None: every station uses the handle's constants)
+        self._bi_consts = None
+        if sc is not None:
+            om = np.stack([stage_weights(self._lib, N_bi, ct, er) for ct, er in zip(sc["cost_type"], sc["exp_rate"])])
+            self._bi_consts = {f: torch.from_numpy(sc[f]).to(self.dev) for f in SCALAR_FIELDS + ("cost_type",)}
+            self._bi_consts["omega"] = torch.from_numpy(om).to(self.dev)
         self.ev = {"s": consts.small_EV_consts, "l": consts.large_EV_consts}
         self.solver = {k: PriceSolver(N_lo, self.ev[k], consts.price_type, device=device) for k in ("s", "l")}
         # total EV capacity of every station (charging_station.py:101), the BiMPC's normalisation
@@ -215,11 +233,16 @@ class ChargingStationFleet:
             self.x.data_ptr(), self.demand.data_ptr(), self.profile_len, t, bi["Mp_s"].data_ptr(),
             bi["Mp_l"].data_ptr(), bi["beta_s"].data_ptr(), bi["beta_l"].data_ptr(), bi["gamma_s"].data_ptr(),
             bi["gamma_l"].data_ptr(), bi["x0"].data_ptr(), bi["demand"].data_ptr(), st))
-        self._ck(lib.bimpc_solve_batch_dev(
-            self.bimpc._h, S, bi["Mp_s"].data_ptr(), bi["Mp_l"].data_ptr(), bi["beta_s"].data_ptr(),
-            bi["beta_l"].data_ptr(), bi["gamma_s"].data_ptr(), bi["gamma_l"].data_ptr(), bi["x0"].data_ptr(),
-            bi["demand"].data_ptr(), bi["w_hat_s"].data_ptr(), bi["w_hat_l"].data_ptr(), bi["u_g"].data_ptr(),
-            bi["status"].data_ptr(), bi["iters"].data_ptr(), bi["obj"].data_ptr(), st))
+        bi_args = (bi["Mp_s"].data_ptr(), bi["Mp_l"].data_ptr(), bi["beta_s"].data_ptr(), bi["beta_l"].data_ptr(),
+                   bi["gamma_s"].data_ptr(), bi["gamma_l"].data_ptr(), bi["x0"].data_ptr(), bi["demand"].data_ptr(),
+                   bi["w_hat_s"].data_ptr(), bi["w_hat_l"].data_ptr(), bi["u_g"].data_ptr(), bi["status"].data_ptr(),
+                   bi["iters"].data_ptr(), bi["obj"].data_ptr(), st)
+        if self._bi_consts is None:
+            self._ck(lib.bimpc_solve_batch_dev(self.bimpc._h, S, *bi_args))
+        else:
+            sc = self._bi_consts
+            self._ck(lib.bimpc_solve_batch_consts_dev(
+                self.bimpc._h, S, *[sc[f].data_ptr() for f in SCALAR_FIELDS + ("cost_type", "omega")], *bi_args))
         for k in ("s", "l"):
             self._ck(lib.fleet_wref_dev(self.device, S, P, N_bi, N_lo, bi["w_hat_" + k].data_ptr(),
                                         self.w[k]["w_ref"].data_ptr(), st))
@@ -356,12 +379,14 @@ class ChargingStationFleet:
     # ------------------------------------------------------------------ logs in the reference schema
     def station_logs(self, s: int) -> dict:
         """``ChargingStation.logs`` of station s (charging_station.py:118-149); its constants carry
-        the station's own number of EVs."""
+        the station's own number of EVs and BiMPC constants."""
         L = {k: v[:, ..., s].cpu().numpy() if v.dim() == 3 else v[:, s].cpu().numpy() for k, v in self.log.items()}
         T = lambda a: np.ascontiguousarray(a.T)  # noqa: E731  [Tf, P] -> [P, Tf]
         consts = self.consts
         if int(self.nevs[s]) != consts.nEVs_per_EV_type:
             consts = dataclasses.replace(consts, nEVs_per_EV_type=int(self.nevs[s]))
+        if self.bimpc_consts[s] is not consts.bimpc_consts:
+            consts = dataclasses.replace(consts, bimpc_consts=self.bimpc_consts[s])
         return {
             "constants": consts,
             "inputs": {"w_s": T(L["w_s"]), "w_l": T(L["w_l"]), "w_hat_s": T(L["w_hat_s"]), "w_hat_l": T(L["w_hat_l"]),

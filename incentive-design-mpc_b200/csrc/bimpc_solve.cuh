@@ -127,6 +127,15 @@ struct BiArgs {
   double* li_scratch;     // [CTAs, global_scratch_doubles()] packed inverse factors of the diagonal blocks [+ state
                           // vectors] (global memory, L2-resident: keeping them out of shared memory lets several
                           // stations share an SM)
+  // Per-station constants, read by bimpc_solve_kernel<true> only (the uniform kernel reads the BiConsts fields and
+  // `omega` above).  Each replaces the BiConsts field of the same name for its station.
+  const double* st_delta;       // [S]
+  const double* st_c_g;         // [S]
+  const double* st_u_g_max;     // [S]
+  const double* st_u_b_max;     // [S]
+  const double* st_x_max;       // [S]
+  const int32_t* st_cost_type;  // [S]
+  const double* st_omega;       // [S,N] stage weights (bimpc_stage_weights of the station's cost type and exp_rate)
 };
 
 // Doubles of per-CTA global scratch: the packed inverse factors of the N diagonal blocks + the state vectors that are
@@ -239,6 +248,11 @@ BI_FN double vec_dot(const double* a, const double* b, int n) {
 }
 
 // One station.  `sm` = scratch_doubles(N, P, T) doubles private to this CTA.
+// PER_STATION: the station's delta, c_g, u_g_max, u_b_max, x_max, cost type and stage weights come from the st_*
+// arrays of `a` instead of `c` and a.omega.  Thread 0 stages the five scalars and the cost type in shared memory (CS,
+// in the spare part of the per-k region) and every use reads them there: they are live through the whole IPM loop and
+// the kernel has no registers left to hold them.  Both modes run the same arithmetic on the same values.
+template <bool PER_STATION = false>
 BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double* sm, double* LI, int tid, int T) {
   const int N = c.N, P = c.P;
   // all 2P partition blocks size the scratch; the loops run over the ACTIVE ones only (see below)
@@ -299,7 +313,7 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
   double* T78 = pk;           pk += N;
   double* DEM = pk;           pk += N;
   double* OM = pk;            pk += N;
-  pk += 9 * N;                          // (spare, keeps the 40 N budget)
+  double* CS = pk;            pk += 9 * N;  // PER_STATION: the station's constants (6 <= 9 N); spare otherwise
   double* AV = pk;            pk += nbmax;  // a = (-m, 1)
   double* LA = pk;            pk += nbmax;  // Linv_{k-1} a
   double* TL = pk;            pk += nbmax;  // T' la
@@ -313,6 +327,11 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
   double* GQ = pk;            pk += Q2max;   // gamma_q
   double* WMX = pk;           pk += Q2max;   // wmax_q
   double* QIDX = pk;          pk += Q2max;   // active block -> partition index (small P, then large P)
+  auto delta = [&] { return PER_STATION ? CS[0] : c.delta; };
+  auto c_g = [&] { return PER_STATION ? CS[1] : c.c_g; };
+  auto u_g_max = [&] { return PER_STATION ? CS[2] : c.u_g_max; };
+  auto u_b_max = [&] { return PER_STATION ? CS[3] : c.u_b_max; };
+  auto x_max = [&] { return PER_STATION ? CS[4] : c.x_max; };
 
   // ---- station data
   const double x0 = a.x0[st_idx];
@@ -335,13 +354,27 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
     int cnt = 0;
     bool finite = isfinite(x0) && isfinite(derr);  // derr: every Mp and beta
     for (int k = 0; k < N; ++k) finite = finite && isfinite(a.demand[(size_t)st_idx * N + k]);
+    int cost_type = c.cost_type;
+    if (PER_STATION) {
+      // The station's constants must pass bimpc_create's checks (>= 0, a known cost type) and be finite, and its
+      // stage weights must be finite; otherwise it gets status 2 like a non-finite input.
+      CS[0] = a.st_delta[st_idx];
+      CS[1] = a.st_c_g[st_idx];
+      CS[2] = a.st_u_g_max[st_idx];
+      CS[3] = a.st_u_b_max[st_idx];
+      CS[4] = a.st_x_max[st_idx];
+      cost_type = a.st_cost_type[st_idx];
+      for (int i = 0; i < 5; ++i) finite = finite && isfinite(CS[i]) && CS[i] >= 0.0;
+      finite = finite && cost_type >= 0 && cost_type <= 2;
+      for (int k = 0; k < N; ++k) finite = finite && isfinite(a.st_omega[(size_t)st_idx * N + k]);
+    }
     for (int q = 0; q < Q2max; ++q) {
       const bool small = q < P;
       const int p = small ? q : q - P;
       const double mp = small ? a.Mp_s[(size_t)st_idx * P + p] : a.Mp_l[(size_t)st_idx * P + p];
       const double th = small ? c.theta_s : c.theta_l;
       const double gq = small ? a.gamma_sm[(size_t)st_idx * P + p] : a.gamma_lm[(size_t)st_idx * P + p];
-      const double aq = c.cost_type == 0 ? (th * mp) * (th * mp) : 1.0;
+      const double aq = cost_type == 0 ? (th * mp) * (th * mp) : 1.0;
       finite = finite && isfinite(gq);
       if (th * mp == 0.0 && (gq == 0.0 || aq == 0.0)) continue;
       MQ[cnt] = th * mp;
@@ -362,13 +395,13 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
   BI_SYNC();
   for (int k = tid; k < N; k += T) {
     DEM[k] = a.demand[(size_t)st_idx * N + k];
-    OM[k] = a.omega[k];
+    OM[k] = PER_STATION ? a.st_omega[(size_t)st_idx * N + k] : a.omega[k];
   }
   BI_SYNC();
   double om_sum = 0.0;
   for (int k = 0; k < N; ++k) om_sum += OM[k];
   double scale_g = 1.0;
-  for (int q = 0; q < Q2; ++q) scale_g = fmax(scale_g, 2.0 * c.delta * AQ[q] * fabs(GQ[q]) * om_sum);
+  for (int q = 0; q < Q2; ++q) scale_g = fmax(scale_g, 2.0 * delta() * AQ[q] * fabs(GQ[q]) * om_sum);
   const double mtot = (double)(2 * QN + 6 * N);
 
   // ---- starting point: box centre, slacks max(h - Gx, 1e-2), multipliers 1
@@ -381,9 +414,9 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
     Z2[i] = 1.0;
   }
   for (int k = tid; k < N; k += T) {
-    U[k] = 0.5 * c.u_g_max;
-    S3[k] = fmax(0.5 * c.u_g_max, 1e-2);
-    S4[k] = fmax(0.5 * c.u_g_max, 1e-2);
+    U[k] = 0.5 * u_g_max();
+    S3[k] = fmax(0.5 * u_g_max(), 1e-2);
+    S4[k] = fmax(0.5 * u_g_max(), 1e-2);
     Z3[k] = Z4[k] = Z5[k] = Z6[k] = Z7[k] = Z8[k] = 1.0;
   }
   BI_SYNC();
@@ -397,10 +430,10 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
     double x = x0;
     for (int j = 0; j <= k; ++j) x += V[j];
     const double e1 = (k == 0) ? derr : 0.0;
-    S5[k] = fmax(V[k] + c.u_b_max - e1, 1e-2);
-    S6[k] = fmax(c.u_b_max - e1 - V[k], 1e-2);
+    S5[k] = fmax(V[k] + u_b_max() - e1, 1e-2);
+    S6[k] = fmax(u_b_max() - e1 - V[k], 1e-2);
     S7[k] = fmax(x - derr, 1e-2);
-    S8[k] = fmax(c.x_max - derr - x, 1e-2);
+    S8[k] = fmax(x_max() - derr - x, 1e-2);
   }
   BI_SYNC();
 
@@ -421,7 +454,7 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
         RDW[q * N + k] = OM[k] * (s - GQ[q]);
       }
       double r = 0.0;
-      const double f = 2.0 * c.delta * AQ[q];
+      const double f = 2.0 * delta() * AQ[q];
       for (int k = N - 1; k >= 0; --k) {
         r += RDW[q * N + k];
         RDW[q * N + k] = f * r;
@@ -456,15 +489,15 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
     }
     for (int k = tid; k < N; k += T) {
       const double u = fmax(U[k], 1e-300);
-      const double rd = 1.7 * c.c_g * pow(u, 0.7) - Z3[k] + Z4[k] + YV[k];
+      const double rd = 1.7 * c_g() * pow(u, 0.7) - Z3[k] + Z4[k] + YV[k];
       RDU[k] = rd;
       r_max = fmax(r_max, fabs(rd));
       const double e1 = (k == 0) ? derr : 0.0;
-      double m = fmax(fabs(S3[k] - U[k]), fabs(U[k] + S4[k] - c.u_g_max));
-      m = fmax(m, fabs(-V[k] + S5[k] - (c.u_b_max - e1)));
-      m = fmax(m, fabs(V[k] + S6[k] - (c.u_b_max - e1)));
+      double m = fmax(fabs(S3[k] - U[k]), fabs(U[k] + S4[k] - u_g_max()));
+      m = fmax(m, fabs(-V[k] + S5[k] - (u_b_max() - e1)));
+      m = fmax(m, fabs(V[k] + S6[k] - (u_b_max() - e1)));
       m = fmax(m, fabs(-XX[k] + S7[k] + derr));
-      m = fmax(m, fabs(XX[k] + S8[k] - (c.x_max - derr)));
+      m = fmax(m, fabs(XX[k] + S8[k] - (x_max() - derr)));
       rp_max = fmax(rp_max, m);
       r_sz += S3[k] * Z3[k] + S4[k] * Z4[k] + S5[k] * Z5[k] + S6[k] * Z6[k] + S7[k] * Z7[k] + S8[k] * Z8[k];
     }
@@ -492,7 +525,7 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
     for (int i = tid; i < QN; i += T) EW[i] = Z1[i] / S1[i] + Z2[i] / S2[i];
     for (int k = tid; k < N; k += T) {
       const double u = fmax(U[k], 1e-300);
-      HU[k] = 1.7 * 0.7 * c.c_g * pow(u, -0.3) + Z3[k] / S3[k] + Z4[k] / S4[k];
+      HU[k] = 1.7 * 0.7 * c_g() * pow(u, -0.3) + Z3[k] / S3[k] + Z4[k] / S4[k];
       D1[k] = Z5[k] / S5[k] + Z6[k] / S6[k];
       D2[k] = Z7[k] / S7[k] + Z8[k] / S8[k];
     }
@@ -532,7 +565,7 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
           XW[i * nb + j] = (i == j) ? 1.0 : 0.0;
           if (j > i) continue;
           double v = rho * AV[i] * AV[j];
-          if (i == j) v += eki + Ek(k + 1, i) + (i < Q2 ? 2.0 * c.delta * AQ[i] * OM[k] : 0.0);
+          if (i == j) v += eki + Ek(k + 1, i) + (i < Q2 ? 2.0 * delta() * AQ[i] * OM[k] : 0.0);
           if (k >= 1) {
             double t0 = 0.0, t1 = 0.0;  // (Linv' Linv)[i][j], i >= j
             int l = i, o = i * (i + 1) / 2;
@@ -684,8 +717,8 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
       };
       for (int k = tid; k < N; k += T) {
         const double e1 = (k == 0) ? derr : 0.0;
-        const double rp5 = -V[k] + S5[k] - (c.u_b_max - e1), rp6 = V[k] + S6[k] - (c.u_b_max - e1);
-        const double rp7 = -XX[k] + S7[k] + derr, rp8 = XX[k] + S8[k] - (c.x_max - derr);
+        const double rp5 = -V[k] + S5[k] - (u_b_max() - e1), rp6 = V[k] + S6[k] - (u_b_max() - e1);
+        const double rp7 = -XX[k] + S7[k] + derr, rp8 = XX[k] + S8[k] - (x_max() - derr);
         const double x5 = (Z5[k] * rp5 - rc_of(S5[k], Z5[k], rp5, -DVA[k])) / S5[k];
         const double x6 = (Z6[k] * rp6 - rc_of(S6[k], Z6[k], rp6, DVA[k])) / S6[k];
         const double x7 = (Z7[k] * rp7 - rc_of(S7[k], Z7[k], rp7, -DXXA[k])) / S7[k];
@@ -708,7 +741,7 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
         DX[i] = -RDW[i] + x1 - x2 + MQ[q] * NU[k];
       }
       for (int k = tid; k < N; k += T) {
-        const double rp3 = S3[k] - U[k], rp4 = U[k] + S4[k] - c.u_g_max;
+        const double rp3 = S3[k] - U[k], rp4 = U[k] + S4[k] - u_g_max();
         const double x3 = (Z3[k] * rp3 - rc_of(S3[k], Z3[k], rp3, -DXUA[k])) / S3[k];
         const double x4 = (Z4[k] * rp4 - rc_of(S4[k], Z4[k], rp4, DXUA[k])) / S4[k];
         BU[k] = -RDU[k] + x3 - x4 - NU[k];
@@ -748,11 +781,11 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
       for (int k = tid; k < N; k += T) {
         const double e1 = (k == 0) ? derr : 0.0;
         ratio(S3[k], Z3[k], S3[k] - U[k], -BU[k], -DXUA[k]);
-        ratio(S4[k], Z4[k], U[k] + S4[k] - c.u_g_max, BU[k], DXUA[k]);
-        ratio(S5[k], Z5[k], -V[k] + S5[k] - (c.u_b_max - e1), -DV[k], -DVA[k]);
-        ratio(S6[k], Z6[k], V[k] + S6[k] - (c.u_b_max - e1), DV[k], DVA[k]);
+        ratio(S4[k], Z4[k], U[k] + S4[k] - u_g_max(), BU[k], DXUA[k]);
+        ratio(S5[k], Z5[k], -V[k] + S5[k] - (u_b_max() - e1), -DV[k], -DVA[k]);
+        ratio(S6[k], Z6[k], V[k] + S6[k] - (u_b_max() - e1), DV[k], DVA[k]);
         ratio(S7[k], Z7[k], -XX[k] + S7[k] + derr, -DXX[k], -DXXA[k]);
-        ratio(S8[k], Z8[k], XX[k] + S8[k] - (c.x_max - derr), DXX[k], DXXA[k]);
+        ratio(S8[k], Z8[k], XX[k] + S8[k] - (x_max() - derr), DXX[k], DXXA[k]);
       }
       block_reduce(RED, tid, T, dummy_s, dummy_m, amin);
       if (pass == 0) {
@@ -772,11 +805,11 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
         for (int k = tid; k < N; k += T) {
           const double e1 = (k == 0) ? derr : 0.0;
           muaff(S3[k], Z3[k], S3[k] - U[k], -BU[k]);
-          muaff(S4[k], Z4[k], U[k] + S4[k] - c.u_g_max, BU[k]);
-          muaff(S5[k], Z5[k], -V[k] + S5[k] - (c.u_b_max - e1), -DV[k]);
-          muaff(S6[k], Z6[k], V[k] + S6[k] - (c.u_b_max - e1), DV[k]);
+          muaff(S4[k], Z4[k], U[k] + S4[k] - u_g_max(), BU[k]);
+          muaff(S5[k], Z5[k], -V[k] + S5[k] - (u_b_max() - e1), -DV[k]);
+          muaff(S6[k], Z6[k], V[k] + S6[k] - (u_b_max() - e1), DV[k]);
           muaff(S7[k], Z7[k], -XX[k] + S7[k] + derr, -DXX[k]);
-          muaff(S8[k], Z8[k], XX[k] + S8[k] - (c.x_max - derr), DXX[k]);
+          muaff(S8[k], Z8[k], XX[k] + S8[k] - (x_max() - derr), DXX[k]);
           DXUA[k] = BU[k];
           DVA[k] = DV[k];
           DXXA[k] = DXX[k];
@@ -812,9 +845,9 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
       }
       for (int k = tid; k < N; k += T) {
         const double e1 = (k == 0) ? derr : 0.0;
-        const double rp3 = S3[k] - U[k], rp4 = U[k] + S4[k] - c.u_g_max;
-        const double rp5 = -V[k] + S5[k] - (c.u_b_max - e1), rp6 = V[k] + S6[k] - (c.u_b_max - e1);
-        const double rp7 = -XX[k] + S7[k] + derr, rp8 = XX[k] + S8[k] - (c.x_max - derr);
+        const double rp3 = S3[k] - U[k], rp4 = U[k] + S4[k] - u_g_max();
+        const double rp5 = -V[k] + S5[k] - (u_b_max() - e1), rp6 = V[k] + S6[k] - (u_b_max() - e1);
+        const double rp7 = -XX[k] + S7[k] + derr, rp8 = XX[k] + S8[k] - (x_max() - derr);
         upd(S3[k], Z3[k], rp3, -BU[k], -DXUA[k]);
         upd(S4[k], Z4[k], rp4, BU[k], DXUA[k]);
         upd(S5[k], Z5[k], rp5, -DV[k], -DVA[k]);
@@ -840,7 +873,7 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
     if (q < P) a.w_hat_s[((size_t)st_idx * P + q) * N + k] = x;
     else a.w_hat_l[((size_t)st_idx * P + (q - P)) * N + k] = x;
   }
-  for (int k = tid; k < N; k += T) a.u_g[(size_t)st_idx * N + k] = fmin(fmax(U[k], 0.0), c.u_g_max);
+  for (int k = tid; k < N; k += T) a.u_g[(size_t)st_idx * N + k] = fmin(fmax(U[k], 0.0), u_g_max());
   if (tid == 0) {
     a.status[st_idx] = status;
     a.iters[st_idx] = it;
@@ -850,12 +883,12 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
     BI_SYNC();
     if (tid == 0) {
       double f = 0.0;
-      for (int k = 0; k < N; ++k) f += c.c_g * pow(fmax(U[k], 0.0), 1.7);
+      for (int k = 0; k < N; ++k) f += c_g() * pow(fmax(U[k], 0.0), 1.7);
       for (int q = 0; q < Q2; ++q) {
         double s = 0.0;
         for (int k = 0; k < N; ++k) {
           s += W[q * N + k];
-          f += c.delta * AQ[q] * OM[k] * (s - GQ[q]) * (s - GQ[q]);
+          f += delta() * AQ[q] * OM[k] * (s - GQ[q]) * (s - GQ[q]);
         }
       }
       a.objective[st_idx] = f;
@@ -865,11 +898,15 @@ BI_FN void solve_station(const BiConsts& c, const BiArgs& a, int st_idx, double*
 }
 
 #ifndef BIMPC_HOSTSIM
+// PER_STATION = false: every station solves with `c` and a.omega.  true: with its own row of the st_* arrays (c
+// supplies N, P and the EV constants).
+template <bool PER_STATION>
 __global__ void __launch_bounds__(kThreads, kMinBlocks) bimpc_solve_kernel(const BiConsts c, const BiArgs a) {
   extern __shared__ double bimpc_smem[];
   for (int s = blockIdx.x; s < a.S; s += gridDim.x) {
-    solve_station(c, a, s, bimpc_smem, a.li_scratch + (size_t)blockIdx.x * global_scratch_doubles(c.N, c.P), threadIdx.x,
-                  blockDim.x);
+    solve_station<PER_STATION>(c, a, s, bimpc_smem,
+                               a.li_scratch + (size_t)blockIdx.x * global_scratch_doubles(c.N, c.P), threadIdx.x,
+                               blockDim.x);
     __syncthreads();
   }
 }

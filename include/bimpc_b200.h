@@ -61,6 +61,43 @@ int bimpc_solve_batch_host(bimpc_t* h, int32_t S, const double* Mp_s, const doub
                            double* w_hat_s, double* w_hat_l, double* u_g, int32_t* status,
                            int32_t* iters, double* objective);
 
+/* Stage weights of the charging cost for horizon N (bimpc.py:255-257): omega[k] =
+ * exp_rate^(k-N+1) for BIMPC_COST_EXP_UNWEIGHTED, 1 otherwise; omega holds N doubles (host).
+ * bimpc_create builds the handle's weights with this function, so a row built here for the
+ * same cost type and exp_rate has the handle's bits.  LOMPC_ERR_CONSTS for an unknown cost
+ * type or exp_rate < 1 (or NaN); LOMPC_ERR_ARG for N < 1 or a NULL omega.               */
+int bimpc_stage_weights(int N, int cost_type, double exp_rate, double* omega);
+
+/* bimpc_solve_batch_dev with one set of BiMPC constants per station: delta, c_g, u_g_max,
+ * u_b_max, x_max [S], cost_type [S] and the stage weights omega [S,N] (a row of
+ * bimpc_stage_weights for the station's cost type and exp_rate).  Same units as the
+ * handle's constants (normalised by each station's own capacity).  These calls IGNORE the
+ * handle's delta, c_g, u_g_max, u_b_max, x_max, cost type and exp_rate; they use its N, P,
+ * theta_s, theta_l, w_max_s, w_max_l and options.  Station s solves exactly as a handle
+ * created with its constants would solve it alone (same bits).  A station whose constants
+ * are negative or not finite, whose cost type is not 0..2 or whose omega row is not finite
+ * gets status BIMPC_ST_BREAKDOWN; the other stations are unaffected.  A NULL pointer among
+ * the constants returns LOMPC_ERR_ARG and launches nothing.  DEVICE pointers, asynchronous
+ * on `stream`.                                                                          */
+int bimpc_solve_batch_consts_dev(bimpc_t* h, int32_t S, const double* delta, const double* c_g,
+                                 const double* u_g_max, const double* u_b_max, const double* x_max,
+                                 const int32_t* cost_type, const double* omega, const double* Mp_s,
+                                 const double* Mp_l, const double* beta_s, const double* beta_l,
+                                 const double* gamma_sm, const double* gamma_lm, const double* x0,
+                                 const double* demand, double* w_hat_s, double* w_hat_l, double* u_g,
+                                 int32_t* status, int32_t* iters, double* objective, void* stream);
+
+/* The same call with HOST pointers, like bimpc_solve_batch_host.  Takes exp_rate [S] in place
+ * of omega and builds each station's weights with bimpc_stage_weights; a station whose cost
+ * type or exp_rate that function refuses gets status BIMPC_ST_BREAKDOWN.                */
+int bimpc_solve_batch_consts_host(bimpc_t* h, int32_t S, const double* delta, const double* c_g,
+                                  const double* u_g_max, const double* u_b_max, const double* x_max,
+                                  const int32_t* cost_type, const double* exp_rate, const double* Mp_s,
+                                  const double* Mp_l, const double* beta_s, const double* beta_l,
+                                  const double* gamma_sm, const double* gamma_lm, const double* x0,
+                                  const double* demand, double* w_hat_s, double* w_hat_l, double* u_g,
+                                  int32_t* status, int32_t* iters, double* objective);
+
 #ifdef __cplusplus
 }
 #endif

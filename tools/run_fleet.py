@@ -4,6 +4,7 @@ Prints one JSON line: per-step latency (CUDA events), p50/p95, price-loop iterat
 
     python tools/run_fleet.py --stations 4096 --steps 96 --chain reference
     python tools/run_fleet.py --stations 4096 --steps 16 --evs-min 100 --evs-max 900 --profile   # mixed sizes
+    python tools/run_fleet.py --stations 4096 --steps 16 --station-mix --profile   # per-station BiMPC constants
 """
 import argparse
 import json
@@ -52,6 +53,27 @@ def station_sizes(S, lo, hi, seed=5):
     return np.random.default_rng(seed).integers(lo, hi + 1, S)
 
 
+def station_mix(base, S, seed=6):
+    """Per-station BiMPC constants from a fixed seed: the base station's battery capacity x_max and rate u_b_max
+    scaled by U(1, 2), its grid limit u_g_max by U(1, 1.5) and its generation cost c_g by U(0.5, 2); the cost type
+    is WEIGHTED, UNWEIGHTED or EXP_UNWEIGHTED (exp_rate 5) with equal probability.  No limit is scaled below the base
+    station's: with the demand of fleet_demand, batteries scaled by 0.80-0.87 left the first step's program too
+    tight for the interior point (status 2)."""
+    import dataclasses
+
+    from chargingstation.bimpc import BiMPCChargingCostType
+    rng = np.random.default_rng(seed)
+    types = list(BiMPCChargingCostType)
+    out = []
+    for _ in range(S):
+        bat = rng.uniform(1.0, 2.0)
+        out.append(dataclasses.replace(base, x_max=base.x_max * bat, u_b_max=base.u_b_max * bat,
+                                       u_g_max=base.u_g_max * rng.uniform(1.0, 1.5),
+                                       c_g=base.c_g * rng.uniform(0.5, 2.0),
+                                       charging_cost_type=types[int(rng.integers(len(types)))]))
+    return out
+
+
 def card():
     """Name and power limit of cuda:0 (the power limit is read, never set)."""
     import subprocess
@@ -75,6 +97,8 @@ def main():
     ap.add_argument("--evs-min", type=int, default=None,
                     help="with --evs-max: station sizes uniform on {min..max}, demand scaled by size / 500")
     ap.add_argument("--evs-max", type=int, default=None)
+    ap.add_argument("--station-mix", action="store_true",
+                    help="per-station BiMPC constants (battery, grid limit, generation cost, cost type), fixed seed")
     ap.add_argument("--partitions", type=int, default=12)
     ap.add_argument("--n-lo", type=int, default=24)
     ap.add_argument("--n-bi", type=int, default=24)
@@ -94,8 +118,9 @@ def main():
     else:
         consts = fleet_consts(args.steps, args.n_lo, args.n_bi, args.evs, args.partitions)
         demand = fleet_demand(consts, args.stations, args.steps, args.n_bi)
+    bimpc_consts = station_mix(consts.bimpc_consts, args.stations) if args.station_mix else None
     fleet = ChargingStationFleet(consts, args.stations, demand=demand, seed=4, rng="device", chain=args.chain,
-                                 max_price_iter=args.max_price_iter, nevs=nevs)
+                                 max_price_iter=args.max_price_iter, nevs=nevs, bimpc_consts=bimpc_consts)
     fleet.profile = args.profile
     for k in ("s", "l"):
         fleet.solver[k].set_loop_mode(args.loop_mode)
@@ -117,7 +142,8 @@ def main():
     out = {**card(), "loop_mode": args.loop_mode,
            "pivot_overflows": [fleet.solver[k].last_pivot_overflows() for k in ("s", "l")],
            "config": f"{args.stations} stations x ({sizes}) EVs, P={args.partitions}, N_lo={args.n_lo}, "
-                     f"N_bi={args.n_bi}, {args.steps} closed-loop steps, chain={args.chain}",
+                     f"N_bi={args.n_bi}, {args.steps} closed-loop steps, chain={args.chain}"
+                     f"{', per-station BiMPC constants' if args.station_mix else ''}",
            "step_ms_p50": float(np.median(ms)), "step_ms_p95": float(np.percentile(ms, 95)),
            "step_ms_first": float(ms[0]), "step_ms_mean": float(ms.mean()), "wall_ms_p50": float(np.median(wall)),
            "price_loop_iters_per_step": fleet.price_loop_iters,
@@ -129,6 +155,16 @@ def main():
     out["evs_per_type"] = {"total": int(fleet.B), "mean": float(fleet.nevs.mean()), "min": int(fleet.nevs.min()),
                            "p50": float(np.median(fleet.nevs)), "p95": float(np.percentile(fleet.nevs, 95)),
                            "max": int(fleet.nevs.max())}
+    st = log["bimpc_status"].cpu().numpy()
+    out["bimpc_status_counts"] = {str(v): int((st == v).sum()) for v in np.unique(st)}
+    bc = fleet.bimpc_consts
+    q = lambda v: {"min": float(np.min(v)), "p50": float(np.median(v)), "max": float(np.max(v))}  # noqa: E731
+    out["bimpc_consts"] = {f: q([getattr(c, f) for c in bc]) for f in ("x_max", "u_b_max", "u_g_max", "c_g", "delta")}
+    out["bimpc_consts"]["cost_types"] = {t: sum(c.charging_cost_type.name == t for c in bc)
+                                         for t in sorted({c.charging_cost_type.name for c in bc})}
+    it = log["bimpc_iters"].cpu().numpy()
+    out["bimpc_iters_by_cost_type"] = {t: float(it[:, [c.charging_cost_type.name == t for c in bc]].mean())
+                                       for t in out["bimpc_consts"]["cost_types"]}
     if args.profile:
         out["phase_ms_median"] = {k: float(np.median([d[k] for d in fleet.phase_ms])) for k in fleet.phase_ms[0]}
         out["phase_ms_p95"] = {k: float(np.percentile([d[k] for d in fleet.phase_ms], 95)) for k in fleet.phase_ms[0]}
